@@ -9,10 +9,12 @@ partitioned across ranks (weak scaling, no collective on the step path; only the
 are reduced once, after the timed region).
 
   python bench.py [--gpus N] [--steps K] [--warmup W]        # this repo's CUDA path
+  python bench.py ... --dump-outputs DIR                     # + obs / reward / done of the last timed step as .npy
   python bench.py --impl reference ...                       # the reference DLL on the host cores
 Under torchrun (N > 1) one rank per GPU; rank 0 prints ONE JSON line.
 """
 import argparse
+import atexit
 import json
 import math
 import multiprocessing as mp
@@ -62,6 +64,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits",
                                           "-lms", "100", "-i", str(self.idx)], stdout=subprocess.PIPE,
                                          stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)  # no sampler outlives the benchmark, even when a step raises
             threading.Thread(target=self._pump, daemon=True).start()
         except Exception:
             self.proc = None
@@ -328,6 +331,8 @@ def run_cuda(args, rank, local_rank, world):
     launches0 = eng.launch_count
     t_wall0 = time.time()
     ms_total, per_launch_ms = timed_pass(eng, args.steps)        # THE timed region: exactly args.steps steps
+    # what the last timed step handed back, copied before the repeats below step the envs further
+    dumped = {"obs": obs.cpu(), "reward": rew.cpu(), "done": done.cpu()} if args.dump_outputs and rank == 0 else None
     launches = eng.launch_count - launches0
     stats_timed = eng.episode_stats()                              # episodes finished inside the timed region
     # clock samples need >= 0.5 s under load (nvidia-smi samples every 100 ms; 20 steps last 6 ms): the same timed pass is
@@ -494,6 +499,8 @@ def run_cuda(args, rank, local_rank, world):
             line["cpu_baseline"] = info
         except Exception as e:  # the CPU leg must never hide the GPU number
             line["cpu_baseline"] = {"value": None, "unit": UNIT, "cores": os.cpu_count(), "kind": "error", "sample": repr(e)}
+    if dumped is not None:
+        _dump_outputs(args.dump_outputs, dumped, np.float32 if dtype == E.F32 else np.float64)
     _emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -539,6 +546,17 @@ def _vecenv_rate(n, K, device):
     return out
 
 
+def _dump_outputs(out_dir, arrays, np_dtype):
+    """--dump-outputs: every array of the last timed step as <out_dir>/<name>.npy in the handle's float type (done flags
+    as 0 / 1), so that two builds can be compared output for output.  The largest configuration writes 20 MiB."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    outs = {name: t.numpy().astype(np_dtype) for name, t in arrays.items()}
+    assert sum(a.nbytes for a in outs.values()) <= 64 << 20
+    for name, a in outs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def _emit(line):
     """The ONE JSON line goes to the real stdout; everything else a library prints (NCCL banner ...) to stderr."""
     os.write(_REAL_STDOUT, (json.dumps(line) + "\n").encode())
@@ -559,7 +577,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--config", default="fp32_1M_K10", choices=sorted(CONFIGS),
                     help="fp32_1M_K10 = BASELINE configs[2], the configuration the metric is quoted on (default)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write obs, reward and done of the last timed step as DIR/<name>.npy (the envs of GPU 0; the "
+                         "inputs are seeded, so equal arguments give equal inputs)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs applies to --impl cuda")
     rank = int(os.environ.get("RANK", 0))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
@@ -571,6 +594,8 @@ def main():
         cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={args.gpus}",
                "--master-addr", "127.0.0.1", "--master-port", str(29400 + os.getpid() % 500), os.path.abspath(__file__),
                "--gpus", str(args.gpus), "--steps", str(args.steps), "--warmup", str(args.warmup), "--config", args.config]
+        if args.dump_outputs:
+            cmd += ["--dump-outputs", args.dump_outputs]
         sys.exit(subprocess.call(cmd))
     run_cuda(args, rank, local_rank, world)
 

@@ -2,7 +2,7 @@
 """Golden trajectories of the ENV LAYER produced by the reference's own Python -- /root/reference/env/ctrl_env.py,
 core/controller.py and core/model.py, unmodified, imported from where they lie -- on top of the reference DLL's own
 machine code (oracle/refpy.py, oracle/_ref/model_simple.so).  Needs /root/reference: run in the build container;
-the output tests/golden/env_golden_refpy.npz is committed and travels to the GPU box.
+the output tests/golden/env_golden_refpy.npz + env_golden_refpy_2.npz is committed; the tests read only that.
 
 For every configuration family of the parity tests, N envs are rolled through more than one episode the way a
 SubprocVecEnv worker does it (`obs, r, done, info = env.step(a)`; on done `env.reset()`), with float64 actions that
@@ -135,7 +135,12 @@ def main():
                       "(unmodified, imported in place) over core/model_simple_win64.dll's own machine code "
                       "(oracle/_ref/model_simple.so); Controller.reset's random/np.random replaced by the Philox stream"}).encode(),
         dtype=np.uint8)
-    np.savez_compressed(os.path.join(HERE, "env_golden_refpy.npz"), **out)
+    # the families with a PID in the loop (ctrl_type other than MANUAL) go to a second file, so that neither exceeds 1 MB
+    second = {n for n, kw in FAMILIES.items() if kw.get("ctrl_type", 3) != 3}
+    np.savez_compressed(os.path.join(HERE, "env_golden_refpy.npz"),
+                        **{k: v for k, v in out.items() if k.split("/")[0] not in second})
+    np.savez_compressed(os.path.join(HERE, "env_golden_refpy_2.npz"),
+                        **{k: v for k, v in out.items() if k.split("/")[0] in second})
 
 
 if __name__ == "__main__":

@@ -146,3 +146,26 @@ def test_bench_reference_arm_prints_one_json_line():
         assert k in d, k
     assert d["impl"] == "reference" and d["value"] > 0 and d["e2e"]["h2d_bytes_per_step"] == 0
     assert d["cpu_baseline"]["kind"] in ("reference", "port") and d["cpu_baseline"]["cores"] >= 1
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_repeat_exactly(tmp_path):
+    """bench.py --dump-outputs: obs / reward / done of the last timed step, identical from run to run."""
+    import json
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    dumps = []
+    for run in ("a", "b"):
+        r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--config", "fp64_4096", "--steps", "7",
+                            "--warmup", "1", "--no-cpu-baseline", "--dump-outputs", str(tmp_path / run)],
+                           capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads(r.stdout)["steps"] == 7
+        dumps.append({n: np.load(tmp_path / run / f"{n}.npy") for n in ("obs", "reward", "done")})
+    a, b = dumps
+    assert a["obs"].shape == (4096, 3) and a["reward"].shape == a["done"].shape == (4096,)
+    assert all(x.dtype == np.float64 for x in a.values())
+    assert np.isfinite(a["obs"]).all() and set(np.unique(a["done"])) <= {0.0, 1.0}
+    for n in a:
+        assert np.array_equal(a[n], b[n]), n

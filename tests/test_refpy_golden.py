@@ -1,7 +1,7 @@
 """The env layer pinned to the reference's OWN Python.
 
-tests/golden/env_golden_refpy.npz holds trajectories produced by /root/reference/env/ctrl_env.py + core/controller.py +
-core/model.py themselves (unmodified, imported in place, over the DLL's own machine code; generator:
+tests/golden/env_golden_refpy.npz (+ env_golden_refpy_2.npz) holds trajectories produced by the reference's
+env/ctrl_env.py + core/controller.py + core/model.py themselves (unmodified, imported in place, over the DLL's own machine code; generator:
 tests/golden/make_env_golden_refpy.py, provenance line inside the file).  Checked here:
   * the reference's Controller.reset, fed the Philox stream, lands on exactly the episode the oracle's
     b747o_env_draw_episode draws (distributions AND draw order, every family);
@@ -22,7 +22,10 @@ if HERE not in sys.path:
 
 
 def _golden():
-    g = np.load(os.path.join(HERE, "golden", "env_golden_refpy.npz"))
+    # stored as two files to keep each under 1 MB: the families with a PID in the loop are in the second
+    g = {}
+    for f in ("env_golden_refpy.npz", "env_golden_refpy_2.npz"):
+        g.update(np.load(os.path.join(HERE, "golden", f)))
     meta = json.loads(bytes(g["meta_json"]).decode())
     return g, meta
 
