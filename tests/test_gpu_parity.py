@@ -154,6 +154,20 @@ REW_EDGE = 2e-3
 REW_JUMP = 0.08
 
 
+def _reward_edge(O, cfg_o, ob, t_o, d_o):
+    """Envs whose oracle pitch error sits within REW_EDGE of the CLASSIC reward's r3 threshold in this step (and envs
+    that were just reset, whose reference is gone); all False for the other reward types."""
+    edge = np.zeros(len(d_o), bool)
+    if cfg_o.rew_type == O.REW_CLASSIC and cfg_o.obs_type != O.OBS_MODEL_STATE:
+        dv = t_o[:, 1] * (math.pi if cfg_o.norm_obs else 1.0)
+        vr = np.where(ob.gather("use_PID_CS") >= 1.0, ob.gather("vartheta_zh"), ob.gather("vartheta"))
+        vr = np.where(d_o, np.nan, vr)   # reset envs: the reference of the finished episode is gone
+        vf = np.where(vr != 0, vr, cfg_o.vartheta_max)
+        edge = np.abs(np.abs(dv / vf) - 0.05) <= REW_EDGE
+        edge |= np.isnan(vr)
+    return edge
+
+
 def _f32_bound_rollout(E, O, n, steps, kw, seed, sticky=0):
     """f32 engine against the oracle; returns per-step worst deviations inside the envelope and the bookkeeping the
     bound tests assert on.  Done flags are compared bit for bit for ALL envs, excused or not."""
@@ -164,7 +178,6 @@ def _f32_bound_rollout(E, O, n, steps, kw, seed, sticky=0):
     ob.reset()
     rng = np.random.default_rng(seed)
     amax = 1.0 if cfg_o.norm_act else cfg_o.action_max
-    classic = cfg_o.rew_type == O.REW_CLASSIC
     out = np.zeros(n, bool)                      # env left the envelope in its running episode
     res = dict(obs=np.zeros(n), rew=np.zeros(n), rew_edge=np.zeros(n), obs_all=np.zeros(n), excused=0, total=0, n_done=0,
                edge_steps=0)
@@ -180,15 +193,7 @@ def _f32_bound_rollout(E, O, n, steps, kw, seed, sticky=0):
         inside = _envelope_update(ob, out, d_o)
         eo = (np.abs(term.astype(np.float64) - t_o) / (1.0 + np.abs(t_o))).max(axis=1)   # relative to 1 + |obs|
         er = np.abs(rew.astype(np.float64) - r_o)
-        edge = np.zeros(n, bool)
-        if classic:
-            dv = t_o[:, 1] * (math.pi if cfg_o.norm_obs else 1.0) if cfg_o.obs_type != O.OBS_MODEL_STATE else None
-            if dv is not None:
-                vr = np.where(ob.gather("use_PID_CS") >= 1.0, ob.gather("vartheta_zh"), ob.gather("vartheta"))
-                vr = np.where(d_o, np.nan, vr)   # reset envs: the reference of the finished episode is gone
-                vf = np.where(vr != 0, vr, cfg_o.vartheta_max)
-                edge = np.abs(np.abs(dv / vf) - 0.05) <= REW_EDGE
-                edge |= np.isnan(vr)
+        edge = _reward_edge(O, cfg_o, ob, t_o, d_o)
         res["obs_all"] = np.maximum(res["obs_all"], eo)
         res["obs"] = np.maximum(res["obs"], np.where(inside, eo, 0.0))
         res["rew"] = np.maximum(res["rew"], np.where(inside & ~edge, er, 0.0))
