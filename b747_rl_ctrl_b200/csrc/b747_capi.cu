@@ -86,7 +86,6 @@ extern "C" void b747_philox4x32(const uint32_t ctr[4], const uint32_t key[2], ui
 
 // ---- field table -----------------------------------------------------------------------------
 namespace {
-enum FieldKind { FK_SLOT, FK_STATE0, FK_SIG, FK_TICK, FK_FLAGS, FK_EPIDX, FK_LASTRET, FK_LASTLEN, FK_MXONLY };
 struct FieldDesc { const char* name; FieldKind kind; int row; };
 const std::vector<FieldDesc>& fields() {
   static std::vector<FieldDesc> f;
@@ -746,7 +745,7 @@ static int field_io(b747_handle* h, int field, double* out, const double* in) {
   CU(cudaStreamSynchronize(h->stream));
   const FieldDesc& f = fields()[field];
   const size_t n = (size_t)h->cfg.n_envs, np = (size_t)h->dc.n_pad;
-  if (h->cfg.dtype == B747_F32) return f32_field_io(h->dc, h->s32, (int)f.kind, f.row, f.name, out, in, h->stream) ? fail(B747_ERR_ARG, std::string("field not available on an f32 handle: ") + f.name) : B747_OK;
+  if (h->cfg.dtype == B747_F32) return f32_field_io(h->dc, h->s32, f.kind, f.row, f.name, out, in, h->stream) ? fail(B747_ERR_ARG, std::string("field not available on an f32 handle: ") + f.name) : B747_OK;
   StateF64& s = h->s64;
   std::vector<int> tmp;
   auto io_double = [&](double* dev) -> int {

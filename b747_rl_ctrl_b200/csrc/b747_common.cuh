@@ -119,6 +119,14 @@ struct Episode {
   int use_ctrl, osc;
 };
 
+// An explicit episode of the C ABI (b747_reset_to) in the kernels' form.
+__device__ inline void episode_from_abi(const b747_episode& e, Episode& ep) {
+  for (int k = 0; k < 6; k++) ep.s0[k] = e.state0[k];
+  ep.vref = e.vref_const; ep.href = e.h_ref; ep.use_ctrl = e.use_ctrl; ep.osc = e.oscillating;
+  for (int k = 0; k < 3; k++) { ep.oscA[k] = e.osc_A[k]; ep.oscf[k] = e.osc_f[k]; }
+  for (int k = 0; k < 5; k++) ep.aerr[k] = e.aero_err[k];
+}
+
 // Controller.reset random part (core/controller.py:144-193): distributions and draw order are the
 // reference's; the stream is Philox keyed by (seed, global env id, episode index).
 __device__ inline void draw_episode(const DevCfg& c, uint64_t env, uint32_t epi, Episode& ep) {

@@ -47,7 +47,9 @@ void launch_env_step32(const DevCfg& c, const StateF32& st, const float* actions
 void launch_reset32(const DevCfg& c, const StateF32& st, const uint8_t* mask, const b747_episode* eps, float* obs,
                     cudaStream_t s);
 void launch_defaults32(const DevCfg& c, const StateF32& st, cudaStream_t s);
-int f32_field_io(const DevCfg& c, StateF32& s, int kind, int row, const char* name, double* out, const double* in,
+// Storage kind of a per-env field of b747_get_field / b747_set_field (field table in b747_capi.cu).
+enum FieldKind { FK_SLOT, FK_STATE0, FK_SIG, FK_TICK, FK_FLAGS, FK_EPIDX, FK_LASTRET, FK_LASTLEN, FK_MXONLY };
+int f32_field_io(const DevCfg& c, StateF32& s, FieldKind kind, int row, const char* name, double* out, const double* in,
                  cudaStream_t stream);
 
 void launch_env_step64(const DevCfg& c, const StateF64& st, const double* actions, double* obs, double* rew,

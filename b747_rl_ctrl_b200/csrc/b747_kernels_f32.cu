@@ -33,7 +33,7 @@ static_assert(DG_vref_ret == 5 && FG_misc == 2, "stage_issue copies D groups 0-5
 
 // The tick word of F[FG_misc] also carries the look-up interval indices between launches (no extra HBM bytes): bit 31
 // set = {tick in bits 0-13, indices in bits 14-30}; bit 31 clear = plain tick (episodes beyond 16383 ticks), no indices.
-__device__ __forceinline__ void unpack_tick(uint32_t w, int& tick, uint32_t& ix) {
+__host__ __device__ __forceinline__ void unpack_tick(uint32_t w, int& tick, uint32_t& ix) {
   if (w & 0x80000000u) { tick = (int)(w & 0x3fffu); ix = (w >> 14) & 0x1ffffu; }
   else { tick = (int)w; ix = kIxEmpty; }
 }
@@ -43,10 +43,10 @@ __device__ __forceinline__ uint32_t pack_tick(int tick, uint32_t ix) {
 
 // CSF = false (step kernel, tier 1): the altitude-loop states and h_zh are neither read nor integrated, so they are not
 // carried through the step at all (8 registers); a reset inside the step writes their fresh values (store_mx, full).
+// D, F: the group arrays with `np` envs per group -- the handle's state in HBM, or a warp's staged tile (np = 32).
 template <bool GEN, bool CSF = true>
-__device__ __forceinline__ void load_mx(const StateF32& st, size_t np, int i, RegsMx& r) {
-  const double2* __restrict__ D = st.D;
-  const float4* __restrict__ F = st.F;
+__device__ __forceinline__ void load_mx(const double2* __restrict__ D, const float4* __restrict__ F, size_t np, int i,
+                                        RegsMx& r) {
   double2 d;
   d = D[DG_h_th * np + i]; r.h = d.x; r.th = d.y;
   d = D[DG_V * np + i]; r.Vx = d.x; r.Vy = d.y;
@@ -93,16 +93,10 @@ __device__ __forceinline__ void load_mx(const StateF32& st, size_t np, int i, Re
 // mbarrier.  The copy of tile k+1 is issued as soon as tile k has been read into registers, so the HBM latency of the
 // next tile hides behind the K model steps of the current one and the memory system always has every warp's next
 // tile in flight (ncu r1e: at K = 1 the step was latency-bound at 58 % of the HBM roof with plain loads).
-// Selected per launch (launch_env_step32): on for K <= B747_STAGED_MAX_K substeps, where the step is HBM-latency bound
+// Selected per launch (launch_env_step32): on for K <= kStagedMaxK substeps, where the step is HBM-latency bound
 // (measured round 1, 1 Mi envs: K=1 0.0737 -> 0.0715 ms), off above (K=2 0.090 vs 0.091 ms, K=10 0.283 vs 0.289 ms: the extra
 // shared-memory round trip costs issue slots the compute-bound regime does not have).
-#ifndef B747_L2_PREFETCH
-#define B747_L2_PREFETCH 0  // 1: next tile's state prefetched into L2 while the current one is stepped (measured round 2,
-                            // steady state K = 10: 0.2890 -> 0.2926 ms with it, 0.3150 -> 0.3189 with static tiles: rejected)
-#endif
-#ifndef B747_STAGED_MAX_K
-#define B747_STAGED_MAX_K 1
-#endif
+constexpr int kStagedMaxK = 1;
 constexpr int kStageGroups = 9, kStageBytes = kStageGroups * 512;
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -130,35 +124,6 @@ __device__ __forceinline__ void stage_issue(const StateF32& st, size_t np, int i
   for (int g = 0; g < 6; g++) bulk_g2s(buf + g * 512, st.D + (size_t)g * np + i0, 512, bar);
 #pragma unroll
   for (int g = 0; g < 3; g++) bulk_g2s(buf + (6 + g) * 512, st.F + (size_t)g * np + i0, 512, bar);
-}
-// all lanes: the staged copy of load_mx<false>
-__device__ __forceinline__ void load_mx_staged(const unsigned char* buf, int lane, RegsMx& r) {
-  const double2* D = (const double2*)buf;
-  const float4* F = (const float4*)(buf + 6 * 512);
-  double2 d;
-  d = D[DG_h_th * 32 + lane]; r.h = d.x; r.th = d.y;
-  d = D[DG_V * 32 + lane]; r.Vx = d.x; r.Vy = d.y;
-  d = D[DG_wz_ssi * 32 + lane]; r.wz = d.x; r.ssi = d.y;
-  d = D[DG_ssf_dvi * 32 + lane]; r.ssf = d.x; r.dvi = d.y;
-  d = D[DG_itse_d1 * 32 + lane]; r.itse = d.x; r.d1_u = d.y;
-  d = D[DG_vref_ret * 32 + lane]; r.vref = d.x; r.ep_return = d.y;
-  float4 f;
-  f = F[FG_act * 32 + lane]; r.df_x = f.x; r.df_y = f.y; r.rl_prev = f.z; r.deltaz = f.w;
-  f = F[FG_uh * 32 + lane]; r.uh[0] = f.x; r.uh[1] = f.y; r.uh[2] = f.z; r.uh[3] = f.w;
-  f = F[FG_misc * 32 + lane]; r.sig_upid = f.x; r.d2_u = f.y;
-  uint32_t ix_hint;
-  unpack_tick(__float_as_uint(f.z), r.tick, ix_hint);
-  const unsigned fw = __float_as_uint(f.w);
-  r.flags = (int)(fw & 0xffu); r.ep_idx = fw >> 8;
-  r.csi = r.csf = r.x = 0.0; r.href = B747_DEF_H_ZH;
-#pragma unroll
-  for (int k = 0; k < 3; k++) { r.oscA[k] = 0.0; r.oscf[k] = 0.0; }
-#pragma unroll
-  for (int k = 0; k < 5; k++) r.sumA[k] = 1.0f;
-  r.tf_tp = 0.f; r.sig_vzh = 0.f;
-  r.vartheta = 0.0;
-  r.tc = TabCache{};
-  r.tc.ix = ix_hint;
 }
 
 // `full`: also the groups a step never changes (reference, aero sums, state0) -- reset paths only.
@@ -253,33 +218,19 @@ __device__ __forceinline__ void load_tables32(float4* sT, const float4* __restri
 }
 
 // ------------------------------------------------------------------------------------------
-#ifndef B747_F32_MINBLOCKS
-#define B747_F32_MINBLOCKS 4
-#endif
-#ifndef B747_F32_THREADS
-#define B747_F32_THREADS 128  // threads per block of the tier-0 step kernel (tiers 1, 2: 128)
-#endif
-#ifndef B747_EXT_MINBLOCKS
-#define B747_EXT_MINBLOCKS 3
-#endif
-#ifndef B747_GEN_MINBLOCKS
-#define B747_GEN_MINBLOCKS 3  // measured: 168 registers x 12 warps beats 242 x 8 (0.66 -> 0.52 ms per 1 Mi-env K=10 step)
-#endif
+constexpr int kStepThreads = 128, kStepWarps = kStepThreads / 32;  // threads per block of every step kernel tier
+constexpr int kF32MinBlocks = 4;  // measured: 4 x 128 threads at 126 registers, no spills, beats every other occupancy point
+constexpr int kExtMinBlocks = 3;
+constexpr int kGenMinBlocks = 3;  // measured: 168 registers x 12 warps beats 242 x 8 (0.66 -> 0.52 ms per 1 Mi-env K=10 step)
 // TIER 0: canonical family (LEAN layout); 1: general layout without the altitude loop (other observation layouts,
 // oscillating references, aero disturbance, TF reward); 2: + the altitude loop (СУ PID); 3: + recorder, tracker, signal export.
 // PFA: the next tile's actions are fetched while the current tile is stepped (host-mapped action buffers: a PCIe read
 // has ~2 us of latency, a tile at K = 10 takes ~20 us).
 template <int TIER, int SW = -1, bool STG = false, bool PFA = false>
-#ifdef B747_F32_MAXNREG
-#define B747_STEP_BOUNDS __launch_bounds__(TIER == 0 ? B747_F32_THREADS : 128) __maxnreg__(TIER == 0 ? B747_F32_MAXNREG : 168)
-#else
-#define B747_STEP_BOUNDS __launch_bounds__(TIER == 0 ? B747_F32_THREADS : 128, TIER >= 2 ? B747_GEN_MINBLOCKS : (TIER == 1 ? B747_EXT_MINBLOCKS : B747_F32_MINBLOCKS))
-#endif
-__global__ void B747_STEP_BOUNDS k_env_step32(DevCfg c, MP32 mp, StateF32 st, const float* __restrict__ actions,
-                                                    float* __restrict__ obs_out, float* __restrict__ rew_out,
-                                                    uint8_t* __restrict__ done_out, float* __restrict__ term_obs,
-                                                    float4* __restrict__ out4, uint32_t* __restrict__ done_bits,
-                                                    unsigned int* __restrict__ tile_ctr) {
+__global__ void __launch_bounds__(kStepThreads, TIER >= 2 ? kGenMinBlocks : (TIER == 1 ? kExtMinBlocks : kF32MinBlocks))
+k_env_step32(DevCfg c, MP32 mp, StateF32 st, const float* __restrict__ actions, float* __restrict__ obs_out,
+             float* __restrict__ rew_out, uint8_t* __restrict__ done_out, float* __restrict__ term_obs,
+             float4* __restrict__ out4, uint32_t* __restrict__ done_bits, unsigned int* __restrict__ tile_ctr) {
   // Persistent warps: the launch fills the GPU once (blocks = SMs x resident blocks per SM), the tables are staged into
   // shared memory once per block, and every warp then walks its own stride of 32-env tiles with no block-level
   // synchronisation until the episode statistics are flushed at the very end.
@@ -287,8 +238,8 @@ __global__ void B747_STEP_BOUNDS k_env_step32(DevCfg c, MP32 mp, StateF32 st, co
   constexpr bool STAGED = !GEN && STG;
   __shared__ float4 sT[kFastCells];
   __shared__ double s_stats[4];
-  __shared__ __align__(128) unsigned char sStage[STAGED ? 4 : 1][STAGED ? kStageBytes : 16];
-  __shared__ __align__(8) unsigned long long sBar[8];
+  __shared__ __align__(128) unsigned char sStage[STAGED ? kStepWarps : 1][STAGED ? kStageBytes : 16];
+  __shared__ __align__(8) unsigned long long sBar[kStepWarps];
   const size_t np = (size_t)c.n_pad;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, warps_per_block = blockDim.x >> 5;
   const int n_tiles = (c.env_hi - c.env_lo + 31) >> 5;
@@ -320,15 +271,6 @@ __global__ void B747_STEP_BOUNDS k_env_step32(DevCfg c, MP32 mp, StateF32 st, co
   }
   const int i = c.env_lo + wt * 32 + lane;
   const bool live = i < c.env_hi;
-  if (B747_L2_PREFETCH && !STAGED && wn < n_tiles && (lane & 7) == 0) {
-    // the next tile's state on its way into L2 while this one is stepped: four 128-byte lines per 512-byte group
-    const int in = c.env_lo + wn * 32 + lane;
-    constexpr int ngd = GEN ? (CS ? 11 : 11) : 6, ngf = GEN ? 5 : 3;
-#pragma unroll
-    for (int g = 0; g < ngd; g++) asm volatile("prefetch.global.L2 [%0];" ::"l"(st.D + (size_t)g * np + in));
-#pragma unroll
-    for (int g = 0; g < ngf; g++) asm volatile("prefetch.global.L2 [%0];" ::"l"(st.F + (size_t)g * np + in));
-  }
   bool done = false;
   double ep_ret = 0.0, ep_len = 0.0;
   RegsMx r;
@@ -336,7 +278,8 @@ __global__ void B747_STEP_BOUNDS k_env_step32(DevCfg c, MP32 mp, StateF32 st, co
   if (STAGED) {
     mbar_wait(bar, phase);
     phase ^= 1;
-    load_mx_staged(&sStage[STAGED ? warp : 0][0], lane, r);
+    const unsigned char* tile = &sStage[STAGED ? warp : 0][0];
+    load_mx<false>((const double2*)tile, (const float4*)(tile + 6 * 512), 32, lane, r);
     __syncwarp();  // every lane has read its slots: the buffer can take the next tile
     if (wn < n_tiles) {
       if (lane == 0) stage_issue(st, np, c.env_lo + wn * 32, buf, bar);
@@ -349,7 +292,7 @@ __global__ void B747_STEP_BOUNDS k_env_step32(DevCfg c, MP32 mp, StateF32 st, co
   }
   if (live) {
     if (!STAGED) {
-      load_mx<GEN, CS>(st, np, i, r);
+      load_mx<GEN, CS>(st.D, st.F, np, i, r);
       if (!PFA) a = actions[i];
     }
     if (c.norm_act) a *= (float)c.action_max;
@@ -557,14 +500,10 @@ __global__ void __launch_bounds__(128) k_reset32(DevCfg c, StateF32 st, const ui
   if (mask && !mask[i]) return;
   const size_t np = (size_t)c.n_pad;
   RegsMx r;
-  load_mx<GEN>(st, np, i, r);
+  load_mx<GEN>(st.D, st.F, np, i, r);
   Episode ep;
   if (eps) {
-    const b747_episode& e = eps[i];
-    for (int k = 0; k < 6; k++) ep.s0[k] = e.state0[k];
-    ep.vref = e.vref_const; ep.href = e.h_ref; ep.use_ctrl = e.use_ctrl; ep.osc = e.oscillating;
-    for (int k = 0; k < 3; k++) { ep.oscA[k] = e.osc_A[k]; ep.oscf[k] = e.osc_f[k]; }
-    for (int k = 0; k < 5; k++) ep.aerr[k] = e.aero_err[k];
+    episode_from_abi(eps[i], ep);
   } else if (c.reset_ref_mode == B747_RESET_NONE) {
     episode_from_state_mx(st, np, i, r, ep);
   } else {
@@ -652,20 +591,12 @@ void f32_free(StateF32& s) {
 
 static inline int grid_for(int n, int block) { return (n + block - 1) / block; }
 
-#ifndef B747_DYNAMIC_TILES
-#define B747_DYNAMIC_TILES 1  // 0: static tile stride per warp
-#endif
 constexpr int kTileCtrSlots = 64;
-#ifndef B747_PERSISTENT
-#define B747_PERSISTENT 1  // 0: one 128-env tile per block (grid = all tiles)
-#endif
 // grid of the step kernel: enough blocks to fill every SM at the occupancy of the instantiation that is launched,
 // never more than the tiles need
 template <int TIER, int SW = -1, bool STG = false, bool PFA = false>
 static int step_grid(int n) {
-  constexpr int threads = TIER == 0 ? B747_F32_THREADS : 128;
-  const int need = grid_for(n, threads);
-  if (!B747_PERSISTENT) return need;
+  const int need = grid_for(n, kStepThreads);
   static int resident[64] = {0};  // per device: SMs x blocks per SM
   int dev = 0;
   cudaGetDevice(&dev);
@@ -673,7 +604,7 @@ static int step_grid(int n) {
   if (!resident[dev]) {
     int sms = 0, per_sm = 0;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_env_step32<TIER, SW, STG, PFA>, threads, 0);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_env_step32<TIER, SW, STG, PFA>, kStepThreads, 0);
     resident[dev] = sms > 0 && per_sm > 0 ? sms * per_sm : need;
   }
   return need < resident[dev] ? need : resident[dev];
@@ -692,25 +623,27 @@ void launch_env_step32(const DevCfg& c, const StateF32& st, const float* actions
   const int n = c.env_hi - c.env_lo;
   if (n <= 0) return;
   const bool plain = !st.trace.trk && !st.trace.rec && !st.sig && !c.force_full;
+  const bool lean = plain && f32_is_lean(c);
+  const bool lean_rp = lean && mp.sw == SW_RP;  // the canonical switch setting (use_RP only) as a compile-time constant
+  const bool staged = lean_rp && !prefetch_actions && c.substeps <= kStagedMaxK;  // HBM-bound regime: TMA-staged state
   // tile counter of this launch: one of kTileCtrSlots words, zeroed on the launch stream (launches of one handle may
   // overlap on different streams -- b747_step_host's chunk pipeline -- so consecutive launches take different slots)
   unsigned int* ctr = nullptr;
-  const bool staged = plain && f32_is_lean(c) && mp.sw == SW_RP && !prefetch_actions && c.substeps <= B747_STAGED_MAX_K;
-  if (st.tile_ctr && B747_DYNAMIC_TILES && !staged) {
+  if (st.tile_ctr && !staged) {
     static std::atomic<unsigned> seq{0};
     ctr = st.tile_ctr + (seq.fetch_add(1) % kTileCtrSlots);
     cudaMemsetAsync(ctr, 0, sizeof(unsigned int), s);
   }
 #define B747_LAUNCH(TIER, ...) \
-  k_env_step32<TIER, ##__VA_ARGS__><<<step_grid<TIER, ##__VA_ARGS__>(n), TIER == 0 ? B747_F32_THREADS : 128, 0, s>>>( \
+  k_env_step32<TIER, ##__VA_ARGS__><<<step_grid<TIER, ##__VA_ARGS__>(n), kStepThreads, 0, s>>>( \
       c, mp, st, actions, obs, rew, done, term_obs, out4, done_bits, ctr)
-  if (plain && f32_is_lean(c) && mp.sw == SW_RP && prefetch_actions)  // host-mapped action buffer (b747_step_host_packed)
+  if (lean_rp && prefetch_actions)  // host-mapped action buffer (b747_step_host_packed)
     B747_LAUNCH(0, SW_RP, false, true);
-  else if (plain && f32_is_lean(c) && mp.sw == SW_RP && c.substeps <= B747_STAGED_MAX_K)  // HBM-bound regime: TMA-staged state
+  else if (staged)
     B747_LAUNCH(0, SW_RP, true);
-  else if (plain && f32_is_lean(c) && mp.sw == SW_RP)  // the canonical switch setting (use_RP only) as a compile-time constant
+  else if (lean_rp)
     B747_LAUNCH(0, SW_RP);
-  else if (plain && f32_is_lean(c))
+  else if (lean)
     B747_LAUNCH(0);
   else if (plain && !f32_needs_cs(c) && mp.sw == SW_RP)
     B747_LAUNCH(1, SW_RP);
@@ -745,40 +678,40 @@ const MxField kMxFields[] = {
 };
 }  // namespace
 
-int f32_field_io(const DevCfg& c, StateF32& s, int kind, int row, const char* name, double* out, const double* in,
+int f32_field_io(const DevCfg& c, StateF32& s, FieldKind kind, int row, const char* name, double* out, const double* in,
                  cudaStream_t stream) {
   const size_t n = (size_t)c.n_envs, np = (size_t)c.n_pad;
-  // kinds follow b747_capi.cu: 2 = signal, 3 = tick, 4 = flags, 5 = ep_idx, 6 = last_ret, 7 = last_len
-  if (kind == 2) {
+  if (kind == FK_SIG) {
     if (!s.sig || in) return -1;
     std::vector<float> tmp(n);
     if (cudaMemcpy(tmp.data(), s.sig + (size_t)row * np, sizeof(float) * n, cudaMemcpyDeviceToHost) != cudaSuccess) return -1;
     for (size_t i = 0; i < n; i++) out[i] = tmp[i];
     return 0;
   }
-  if (kind == 6) {
+  if (kind == FK_LASTRET) {
     if (in) return -1;
     return cudaMemcpy(out, s.last_ret, sizeof(double) * n, cudaMemcpyDeviceToHost) != cudaSuccess;
   }
-  if (kind == 7) {
+  if (kind == FK_LASTLEN) {
     if (in) return -1;
     std::vector<int> tmp(n);
     if (cudaMemcpy(tmp.data(), s.last_len, sizeof(int) * n, cudaMemcpyDeviceToHost) != cudaSuccess) return -1;
     for (size_t i = 0; i < n; i++) out[i] = tmp[i];
     return 0;
   }
-  if (kind == 3 || kind == 4 || kind == 5) {
+  if (kind == FK_TICK || kind == FK_FLAGS || kind == FK_EPIDX) {
     std::vector<float4> tmp(n);
     float4* dev = s.F + (size_t)FG_misc * np;
     if (cudaMemcpy(tmp.data(), dev, sizeof(float4) * n, cudaMemcpyDeviceToHost) != cudaSuccess) return -1;
     for (size_t i = 0; i < n; i++) {
-      uint32_t tz, fw;
+      uint32_t tz, fw, ix;
       memcpy(&tz, &tmp[i].z, 4); memcpy(&fw, &tmp[i].w, 4);
-      const int tick = (tz & 0x80000000u) ? (int)(tz & 0x3fffu) : (int)tz;  // unpack_tick
-      if (out) out[i] = kind == 3 ? (double)tick : (kind == 4 ? (double)(fw & 0xffu) : (double)(fw >> 8));
+      int tick;
+      unpack_tick(tz, tick, ix);
+      if (out) out[i] = kind == FK_TICK ? (double)tick : (kind == FK_FLAGS ? (double)(fw & 0xffu) : (double)(fw >> 8));
       else {
-        if (kind == 3) tz = (uint32_t)(int)in[i] & 0x7fffffffu;  // plain tick: the interval hints are dropped
-        else if (kind == 4) fw = (fw & ~0xffu) | ((uint32_t)in[i] & 0xffu);
+        if (kind == FK_TICK) tz = (uint32_t)(int)in[i] & 0x7fffffffu;  // plain tick: the interval hints are dropped
+        else if (kind == FK_FLAGS) fw = (fw & ~0xffu) | ((uint32_t)in[i] & 0xffu);
         else fw = (fw & 0xffu) | ((uint32_t)in[i] << 8);
         memcpy(&tmp[i].z, &tz, 4); memcpy(&tmp[i].w, &fw, 4);
       }

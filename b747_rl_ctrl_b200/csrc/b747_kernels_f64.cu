@@ -180,26 +180,12 @@ __device__ __forceinline__ void load_tables64(double* sP) {
 // ------------------------------------------------------------------------------------------
 // ControllerEnv.step for every env of the handle.
 // ------------------------------------------------------------------------------------------
-#ifndef B747_F64_SMEM_COLD
-#define B747_F64_SMEM_COLD 0  // stash of the fields the model step never reads: no effect (ptxas already keeps them in local memory)
-#endif
-#ifndef B747_F64_MINBLOCKS
-#define B747_F64_MINBLOCKS 2
-#endif
-__global__ void __launch_bounds__(128, B747_F64_MINBLOCKS) k_env_step64(DevCfg c, StateF64 st, const double* __restrict__ actions,
+constexpr int kF64MinBlocks = 2;  // measured: beats 3 / 4 blocks at 168 / 128 registers (1.783 vs 2.04-2.22 ms: spills)
+__global__ void __launch_bounds__(128, kF64MinBlocks) k_env_step64(DevCfg c, StateF64 st, const double* __restrict__ actions,
                                                     double* __restrict__ obs_out, double* __restrict__ rew_out,
                                                     uint8_t* __restrict__ done_out, double* __restrict__ term_obs) {
   __shared__ double sP[kNP];
   __shared__ EpStatsSmem sst;
-#if B747_F64_SMEM_RK
-  __shared__ Rk64Smem srk;
-#define B747_RK_PTR &srk.v[0][threadIdx.x]
-#else
-#define B747_RK_PTR nullptr
-#endif
-#if B747_F64_SMEM_COLD
-  __shared__ struct { double v[12][128]; } scold;
-#endif
   load_tables64(sP);
   const int i = c.env_lo + blockIdx.x * blockDim.x + threadIdx.x;
   const bool live = i < c.env_hi;
@@ -236,18 +222,9 @@ __global__ void __launch_bounds__(128, B747_F64_MINBLOCKS) k_env_step64(DevCfg c
       r.deltaz = dz;
     }
     const bool tracing = st.trace.trk || st.trace.rec;
-#if B747_F64_SMEM_COLD
-    // fields the model step never reads wait in shared memory while the K substeps run (13 doubles = 26 registers of a
-    // kernel that spills at the 255-register limit)
-    double* cold = &scold.v[0][threadIdx.x];
-    cold[0 * 128] = r.sig_upid; cold[1 * 128] = r.sig_vzh; cold[2 * 128] = r.vref; cold[3 * 128] = r.href;
-    cold[4 * 128] = r.oscA[0]; cold[5 * 128] = r.oscA[1]; cold[6 * 128] = r.oscA[2];
-    cold[7 * 128] = r.oscf[0]; cold[8 * 128] = r.oscf[1]; cold[9 * 128] = r.oscf[2];
-    cold[10 * 128] = r.ep_return; cold[11 * 128] = r.tf_tp;
-#endif
 #pragma unroll 1
     for (int k = 0; k < c.substeps; k++) {
-      model_step64(sP, c.mp, r, o, Xs4, B747_RK_PTR);
+      model_step64(sP, c.mp, r, o, Xs4);
       if (tracing) {  // Controller._post_step (core/controller.py:209-228)
         TraceSample ts;
         ts.t = (double)r.tick * kH; ts.U_com = o.U_com; ts.U_PID = o.U_com_PID; ts.deltaz_RP = o.deltaz_RP;
@@ -256,12 +233,6 @@ __global__ void __launch_bounds__(128, B747_F64_MINBLOCKS) k_env_step64(DevCfg c
         trace_model_step(st.trace, np, i, r.tick - 1, ts);
       }
     }
-#if B747_F64_SMEM_COLD
-    r.vref = cold[2 * 128]; r.href = cold[3 * 128];
-    r.oscA[0] = cold[4 * 128]; r.oscA[1] = cold[5 * 128]; r.oscA[2] = cold[6 * 128];
-    r.oscf[0] = cold[7 * 128]; r.oscf[1] = cold[8 * 128]; r.oscf[2] = cold[9 * 128];
-    r.ep_return = cold[10 * 128]; r.tf_tp = cold[11 * 128];
-#endif
     r.sig_upid = o.U_com_PID; r.sig_vzh = o.vartheta_zh;
     const double time = (double)r.tick * kH;
     if (st.trace.trk) {  // Controller.quality of the running episode
@@ -305,9 +276,6 @@ __global__ void __launch_bounds__(128, B747_F64_MINBLOCKS) k_env_step64(DevCfg c
 // Model.step x n_steps (core/model.py:247-250): no action law, no reward.
 __global__ void __launch_bounds__(128) k_model_step64(DevCfg c, StateF64 st, int n_steps) {
   __shared__ double sP[kNP];
-#if B747_F64_SMEM_RK
-  __shared__ Rk64Smem srk;
-#endif
   load_tables64(sP);
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= c.n_envs) return;
@@ -317,7 +285,7 @@ __global__ void __launch_bounds__(128) k_model_step64(DevCfg c, StateF64 st, int
   Pass64 o;
   double Xs4[16];
 #pragma unroll 1
-  for (int k = 0; k < n_steps; k++) model_step64(sP, c.mp, r, o, Xs4, B747_RK_PTR);
+  for (int k = 0; k < n_steps; k++) model_step64(sP, c.mp, r, o, Xs4);
   r.sig_upid = o.U_com_PID; r.sig_vzh = o.vartheta_zh;
   if (st.sig) export_signals64(st.sig, np, i, r, o, Xs4, (double)r.tick * kH);
   store_regs64(st.slots, st.tick, st.flags, st.ep_idx, np, i, r);
@@ -336,11 +304,7 @@ __global__ void __launch_bounds__(128) k_reset64(DevCfg c, StateF64 st, const ui
   load_regs64(st.slots, st.tick, st.flags, st.ep_idx, np, i, r);
   Episode ep;
   if (eps) {
-    const b747_episode& e = eps[i];
-    for (int k = 0; k < 6; k++) ep.s0[k] = e.state0[k];
-    ep.vref = e.vref_const; ep.href = e.h_ref; ep.use_ctrl = e.use_ctrl; ep.osc = e.oscillating;
-    for (int k = 0; k < 3; k++) { ep.oscA[k] = e.osc_A[k]; ep.oscf[k] = e.osc_f[k]; }
-    for (int k = 0; k < 5; k++) ep.aerr[k] = e.aero_err[k];
+    episode_from_abi(eps[i], ep);
   } else if (c.reset_ref_mode == B747_RESET_NONE) {
     episode_from_slots(st.slots, np, i, r, ep);
   } else {

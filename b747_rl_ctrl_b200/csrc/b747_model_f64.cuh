@@ -266,31 +266,16 @@ __device__ __forceinline__ void pass64(const double* __restrict__ P, const Model
 
 // model_simple_step: major pass + update + ode4.  On return r.X holds the post-update states,
 // `o` and Xs4 the stage-4 pass (= what the DLL's exported signals show, SURVEY.md 0.4).
-// B747_F64_SMEM_RK = 1: the RK4 sum and the step's initial state (32 doubles per env) live in shared memory instead of
-// registers (`rk` = this thread's column of a [32][128] block array).  A build switch for measurements only.
-#ifndef B747_F64_SMEM_RK
-#define B747_F64_SMEM_RK 0  // measured round 2 (256 Ki envs, K = 10, steady state): 1.783 ms with registers, 1.824 ms with the
-                            // shared-memory arrays; 3 / 4 blocks per SM (168 / 128 registers): 2.14-2.22 / 2.04 ms -- rejected
-#endif
-struct Rk64Smem { double v[32][128]; };
-
 __device__ __forceinline__ void model_step64(const double* __restrict__ P, const ModelParams& mp, Regs64& r, Pass64& o,
-                                             double Xs4[16], double* __restrict__ rk = nullptr) {
+                                             double Xs4[16]) {
   const int n = r.tick;
   const double t0 = (double)n * kH, tnew = (double)(n + 1) * kH;
   const double t_prev = (double)(n - 1) * kH;
   Held64 hd;
   double f[16];
-#if B747_F64_SMEM_RK
-#define Y_(i) rk[(i) * 128]
-#define ACC_(i) rk[(16 + (i)) * 128]
-#else
-  double acc_[16], y_[16];
-#define Y_(i) y_[i]
-#define ACC_(i) acc_[i]
-#endif
+  double acc[16], y[16];
 #pragma unroll
-  for (int i = 0; i < 16; i++) { Y_(i) = r.X[i]; Xs4[i] = r.X[i]; }
+  for (int i = 0; i < 16; i++) { y[i] = r.X[i]; Xs4[i] = r.X[i]; }
   const double hh = kH, temp = 0.5 * hh;
   const double th = t0 + temp;
   double u_n = 0.0;
@@ -308,22 +293,20 @@ __device__ __forceinline__ void model_step64(const double* __restrict__ P, const
       r.d1_u = o.dv; r.d2_u = o.dv_dt;
       u_n = o.U_com;  // pushed into the ring; first needed as uh[3] of the NEXT step
 #pragma unroll
-      for (int i = 0; i < 16; i++) ACC_(i) = f[i];
+      for (int i = 0; i < 16; i++) acc[i] = f[i];
     } else if (s < 3) {
 #pragma unroll
-      for (int i = 0; i < 16; i++) ACC_(i) = ACC_(i) + 2.0 * f[i];
+      for (int i = 0; i < 16; i++) acc[i] = acc[i] + 2.0 * f[i];
     }
     if (s < 3) {
       const double c = (s == 2) ? hh : temp;
 #pragma unroll
-      for (int i = 0; i < 16; i++) Xs4[i] = Y_(i) + c * f[i];
+      for (int i = 0; i < 16; i++) Xs4[i] = y[i] + c * f[i];
     }
   }
   const double h6 = hh / 6.0;
 #pragma unroll
-  for (int i = 0; i < 16; i++) r.X[i] = Y_(i) + h6 * (ACC_(i) + f[i]);
-#undef Y_
-#undef ACC_
+  for (int i = 0; i < 16; i++) r.X[i] = y[i] + h6 * (acc[i] + f[i]);
   r.uh[0] = r.uh[1]; r.uh[1] = r.uh[2]; r.uh[2] = r.uh[3]; r.uh[3] = u_n;
   r.tick = n + 1;
 }

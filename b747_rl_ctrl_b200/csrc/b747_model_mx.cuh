@@ -43,22 +43,10 @@
 #include "b747_poly.h"
 #include "b747_tables.h"
 
-#ifndef B747_UNROLL_STAGES
-#define B747_UNROLL_STAGES 1  // 1: the four diagram passes of a model step are specialised copies; 0: one rolled loop
-#endif
-
 namespace b747 {
 
-// packed FP32 FMA on a register pair; B747_PAIR_* = 0 falls back to two scalar FMAs (build switches for measurements)
-#ifndef B747_PAIR_RK
-#define B747_PAIR_RK 1
-#endif
-#ifndef B747_PAIR_TAB
-#define B747_PAIR_TAB 1
-#endif
-__device__ __forceinline__ float2 fma2(float2 a, float2 b, float2 c, bool packed) {
-  return packed ? __ffma2_rn(a, b, c) : make_float2(fmaf(a.x, b.x, c.x), fmaf(a.y, b.y, c.y));
-}
+// packed FP32 FMA on a register pair (one FFMA2)
+__device__ __forceinline__ float2 fma2(float2 a, float2 b, float2 c) { return __ffma2_rn(a, b, c); }
 
 __host__ __device__ constexpr double Pc(int i) {
   constexpr double a[kNP] = B747_P_INIT;
@@ -182,7 +170,7 @@ __device__ __forceinline__ float bilinear(const float4 c, float d0, float d1) {
 // two tables at once: three FFMA2 (sm_100 packed FP32; the scalar offsets ride as broadcast operands)
 __device__ __forceinline__ float2 bilinear2(const float2 p[4], float d0, float2 d1) {
   const float2 d00 = make_float2(d0, d0);
-  return fma2(fma2(p[3], d00, p[2], B747_PAIR_TAB), d1, fma2(p[1], d00, p[0], B747_PAIR_TAB), B747_PAIR_TAB);
+  return fma2(fma2(p[3], d00, p[2]), d1, fma2(p[1], d00, p[0]));
 }
 
 // Cold paths.  An operand left its cached interval (or nothing is cached yet); interval indices move incrementally (an
@@ -344,8 +332,8 @@ __device__ __forceinline__ void pass32(const float4* __restrict__ sT, const MP32
     const float cd = fmaf(d2, fmaf(d2, 4.16666667e-2f, -0.5f), 1.0f);
     // (sin, cos)(theta0 + dl) = (sin, cos) cd + (cos, -sin) sd: one packed multiply and one packed FMA
     const float2 cdd = make_float2(cd, cd), sdd = make_float2(sd, sd);
-    const float2 t = B747_PAIR_RK ? __fmul2_rn(tg.cn, sdd) : make_float2(tg.cn.x * sd, tg.cn.y * sd);
-    const float2 rot = fma2(tg.sc, cdd, t, B747_PAIR_RK);
+    const float2 t = __fmul2_rn(tg.cn, sdd);
+    const float2 rot = fma2(tg.sc, cdd, t);
     sn = rot.x;
     cs = fabsf(rot.y);  // the folded pitch stays within +-90 deg: cos >= 0 (a half step may cross the fold)
   }
@@ -409,7 +397,7 @@ __device__ __forceinline__ void pass32(const float4* __restrict__ sT, const MP32
   if (__builtin_expect(missMAH | axis_miss(dC, tc.wC), 0))
     tab_update(sT, Mach, alpha, h, cy_gain, missMAH, tc, dM, dA, dH, cm, dC);
   const float2 dMM = make_float2(dM, dM);
-  const float2 ix = fma2(tc.cxA, dMM, tc.cxB, B747_PAIR_TAB), id = fma2(tc.dcA, dMM, tc.dcB, B747_PAIR_TAB);  // inner terms (c3 dM + c2, c1 dM + c0)
+  const float2 ix = fma2(tc.cxA, dMM, tc.cxB), id = fma2(tc.dcA, dMM, tc.dcB);  // inner terms (c3 dM + c2, c1 dM + c0)
   const float CYa = cm.x;
   // cx = P126 CXa and dcm = P217 P150 dCm: the cells carry the diagram's gains (b747_tables.h)
   float mz = cm.y, cx = fmaf(ix.x, dC, ix.y), dcm = fmaf(id.x, dH, id.y);
@@ -531,11 +519,7 @@ __device__ __forceinline__ void model_step32(const float4* __restrict__ sT, cons
   float u_n = 0.f;
   AtmoMx at;
   TrigMx tg;
-#if B747_UNROLL_STAGES
 #pragma unroll
-#else
-#pragma unroll 1
-#endif
   for (int s = 0; s < 4; s++) {
     const bool ends = (s == 0 || s == 3);
     const float t_f = s == 0 ? t0f : (s == 3 ? t0f + hh : t0f + hhalf);
@@ -561,8 +545,8 @@ __device__ __forceinline__ void model_step32(const float4* __restrict__ sT, cons
     } else {
       const float w = ends ? 1.f : 2.f;
       const float2 ww = make_float2(w, w);
-      aHT = fma2(ww, XVW, aHT, B747_PAIR_RK); aVW = fma2(ww, fVW, aVW, B747_PAIR_RK); aXI = fma2(ww, fXI, aXI, B747_PAIR_RK);
-      aFD = fma2(ww, fFD, aFD, B747_PAIR_RK);
+      aHT = fma2(ww, XVW, aHT); aVW = fma2(ww, fVW, aVW); aXI = fma2(ww, fXI, aXI);
+      aFD = fma2(ww, fFD, aFD);
       a_itse = fmaf(w, f_itse, a_itse);
       if (want_x) a_x = fmaf(w, XXI.x, a_x);
     }
@@ -580,7 +564,7 @@ __device__ __forceinline__ void model_step32(const float4* __restrict__ sT, cons
       }
       const float2 cc = make_float2(cf, cf);
       X_h = fmaf(cf, f_h, y_h);
-      XVW = fma2(cc, fVW, yVW, B747_PAIR_RK); XXI = fma2(cc, fXI, yXI, B747_PAIR_RK);
+      XVW = fma2(cc, fVW, yVW); XXI = fma2(cc, fXI, yXI);
       X_ssf = fmaf(cf, f_ssf, y_ssf);
       if (CS) {
         X_csi = fma(cfd, f_csi, r.csi); X_csf = fma(cfd, f_csf, r.csf);
