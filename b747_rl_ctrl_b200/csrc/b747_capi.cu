@@ -42,7 +42,7 @@ struct b747_handle {
   // it the copy engines hold the link better (7.3e9 against 6.8e9, profiles/r2_hostlink_probe.md).  Results are identical.
   int auto_calls = 0, auto_choice = -1;
   double auto_sec[2] = {0.0, 0.0};
-  // b747_step_host pipeline: copy-in / second compute / copy-out streams and per-chunk events (created on first use)
+  // host-step pipeline (issue_pipeline): copy-in / second compute / copy-out streams and per-chunk events
   cudaStream_t s_in = nullptr, s_aux = nullptr, s_out = nullptr, s_cap = nullptr;
   std::vector<cudaEvent_t> ev_in, ev_k;
   cudaEvent_t ev_start = nullptr, ev_done = nullptr;
@@ -382,33 +382,24 @@ extern "C" int b747_reset_to(b747_handle* h, const b747_episode* eps, void* obs_
   return b747_reset_to_masked(h, eps, nullptr, obs_dev);
 }
 
+// One env step of envs [lo, hi) on stream s with the step kernel of the handle's dtype.
+static void step_range(b747_handle* h, int lo, int hi, const void* act, void* obs, void* rew, uint8_t* done, void* term,
+                       cudaStream_t s) {
+  DevCfg dc = h->dc;
+  dc.env_lo = lo; dc.env_hi = hi;
+  if (h->cfg.dtype == B747_F64)
+    launch_env_step64(dc, h->s64, (const double*)act, (double*)obs, (double*)rew, done, (double*)term, s);
+  else
+    launch_env_step32(dc, h->s32, (const float*)act, (float*)obs, (float*)rew, done, (float*)term, s);
+  h->launches++;
+}
+
 extern "C" int b747_step(b747_handle* h, const void* act, void* obs, void* rew, uint8_t* done, void* term) {
   if (!h || !act || !obs || !rew || !done) return fail(B747_ERR_ARG, "null argument");
   if (!h->cfg.env_layer) return fail(B747_ERR_STATE, "handle was created with env_layer=0; use b747_model_step");
   CU(cudaSetDevice(h->cfg.device));
-  if (h->cfg.dtype == B747_F64)
-    launch_env_step64(h->dc, h->s64, (const double*)act, (double*)obs, (double*)rew, done, (double*)term, h->stream);
-  else
-    launch_env_step32(h->dc, h->s32, (const float*)act, (float*)obs, (float*)rew, done, (float*)term, h->stream);
-  h->launches++;
+  step_range(h, 0, h->cfg.n_envs, act, obs, rew, done, term, h->stream);
   CU(cudaGetLastError());
-  return B747_OK;
-}
-
-// One env step with HOST buffers.  Small batches: copy in, one launch, copy out.  Large batches run as a pipeline over
-// env chunks -- actions of chunk c+1 go up and results of chunk c-1 come down (PCIe is full duplex, the copy engines run
-// beside the SMs) while chunk c is stepped; chunks alternate between two compute streams so that the tail wave of one
-// overlaps the head of the next.  Environments are independent, so chunking cannot change any result.
-static int step_chunk(b747_handle* h, int lo, int hi, bool term, cudaStream_t s) {
-  DevCfg dc = h->dc;
-  dc.env_lo = lo; dc.env_hi = hi;
-  if (h->cfg.dtype == B747_F64)
-    launch_env_step64(dc, h->s64, (const double*)h->d_act, (double*)h->d_obs, (double*)h->d_rew, h->d_done,
-                      term ? (double*)h->d_term : nullptr, s);
-  else
-    launch_env_step32(dc, h->s32, (const float*)h->d_act, (float*)h->d_obs, (float*)h->d_rew, h->d_done,
-                      term ? (float*)h->d_term : nullptr, s);
-  h->launches++;
   return B747_OK;
 }
 
@@ -418,63 +409,20 @@ extern "C" int b747_set_host_chunks(b747_handle* h, int n_chunks) {
   return B747_OK;
 }
 
-// Enqueue one pipelined env step: forks from the handle's stream (copy-in, second compute and copy-out streams) and joins
-// back into it, so the whole step is ordered like a single operation on that stream -- and can be stream-captured.
-static int issue_pipeline(b747_handle* h, cudaStream_t origin, const void* act, void* obs, void* rew, uint8_t* done,
-                          void* term, int chunks, size_t per) {
-  const size_t n = (size_t)h->cfg.n_envs, es = h->elem(), od = (size_t)h->dc.obs_dim;
-  // everything queued on the handle's stream so far (resets, device-side steps) comes first
-  CU(cudaEventRecord(h->ev_start, origin));
-  CU(cudaStreamWaitEvent(h->s_in, h->ev_start, 0));
-  CU(cudaStreamWaitEvent(h->s_aux, h->ev_start, 0));
-  const char* a8 = (const char*)act;
-  char *o8 = (char*)obs, *r8 = (char*)rew, *t8 = (char*)term;
-  for (int c = 0; c < chunks; c++) {
-    const size_t lo = (size_t)c * per, hi = std::min(n, lo + per), m = hi - lo;
-    CU(cudaMemcpyAsync((char*)h->d_act + es * lo, a8 + es * lo, es * m, cudaMemcpyHostToDevice, h->s_in));
-    CU(cudaEventRecord(h->ev_in[c], h->s_in));
-    cudaStream_t sc = (c & 1) ? h->s_aux : origin;
-    CU(cudaStreamWaitEvent(sc, h->ev_in[c], 0));
-    step_chunk(h, (int)lo, (int)hi, term != nullptr, sc);
-    CU(cudaGetLastError());
-    CU(cudaEventRecord(h->ev_k[c], sc));
-    CU(cudaStreamWaitEvent(h->s_out, h->ev_k[c], 0));
-    CU(cudaMemcpyAsync(o8 + es * od * lo, (char*)h->d_obs + es * od * lo, es * od * m, cudaMemcpyDeviceToHost, h->s_out));
-    CU(cudaMemcpyAsync(r8 + es * lo, (char*)h->d_rew + es * lo, es * m, cudaMemcpyDeviceToHost, h->s_out));
-    CU(cudaMemcpyAsync(done + lo, h->d_done + lo, m, cudaMemcpyDeviceToHost, h->s_out));
-    if (term) CU(cudaMemcpyAsync(t8 + es * od * lo, (char*)h->d_term + es * od * lo, es * od * m, cudaMemcpyDeviceToHost, h->s_out));
-  }
-  // join: the copy-out stream has seen every chunk's kernel (and through them every copy-in)
-  CU(cudaEventRecord(h->ev_done, h->s_out));
-  CU(cudaStreamWaitEvent(origin, h->ev_done, 0));
-  return B747_OK;
+// Number of chunks of a host step, `per` envs each (whole thread blocks; the last chunk is ragged).  Without
+// can_pipeline the step is one chunk.
+static int plan_chunks(const b747_handle* h, bool can_pipeline, size_t& per) {
+  const size_t n = (size_t)h->cfg.n_envs;
+  int chunks = 1;
+  if (can_pipeline) chunks = h->host_chunks ? h->host_chunks : (n >= ((size_t)1 << 17) ? 4 : 1);  // measured: 4 beats 8 and 2
+  per = ((n + chunks - 1) / chunks + 127) / 128 * 128;
+  return (int)((n + per - 1) / per);  // whole-block rounding can empty the last chunks
 }
 
-static bool is_pinned(const void* p) {
-  cudaPointerAttributes a;
-  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
-  return a.type == cudaMemoryTypeHost;
-}
-
-extern "C" int b747_step_host(b747_handle* h, const void* act, void* obs, void* rew, uint8_t* done, void* term) {
-  if (!h || !act || !obs || !rew || !done) return fail(B747_ERR_ARG, "null argument");
-  if (!h->cfg.env_layer) return fail(B747_ERR_STATE, "handle was created with env_layer=0; use b747_model_step");
-  CU(cudaSetDevice(h->cfg.device));
-  const size_t n = (size_t)h->cfg.n_envs, es = h->elem(), od = (size_t)h->dc.obs_dim;
-  int chunks = h->host_chunks ? h->host_chunks : (n >= ((size_t)1 << 17) ? 4 : 1);  // measured: 4 beats 8 and 2
-  const size_t per = ((n + chunks - 1) / chunks + 127) / 128 * 128;  // whole thread blocks per chunk
-  chunks = (int)((n + per - 1) / per);  // whole-block rounding can empty the last chunks
-  if (chunks == 1) {
-    CU(cudaMemcpyAsync(h->d_act, act, es * n, cudaMemcpyHostToDevice, h->stream));
-    step_chunk(h, 0, (int)n, term != nullptr, h->stream);
-    CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(obs, h->d_obs, es * n * od, cudaMemcpyDeviceToHost, h->stream));
-    CU(cudaMemcpyAsync(rew, h->d_rew, es * n, cudaMemcpyDeviceToHost, h->stream));
-    CU(cudaMemcpyAsync(done, h->d_done, n, cudaMemcpyDeviceToHost, h->stream));
-    if (term) CU(cudaMemcpyAsync(term, h->d_term, es * n * od, cudaMemcpyDeviceToHost, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
-    return B747_OK;
-  }
+// The pipeline's copy-in / second compute / copy-out streams, the capture stream, the fork / join events and one pair of
+// events per chunk, created on first use (b747_destroy releases them).
+static int pipeline_resources(b747_handle* h, int chunks) {
+  if (chunks < 2) return B747_OK;
   if (!h->s_in) {
     CU(cudaStreamCreateWithFlags(&h->s_in, cudaStreamNonBlocking));
     CU(cudaStreamCreateWithFlags(&h->s_aux, cudaStreamNonBlocking));
@@ -489,9 +437,86 @@ extern "C" int b747_step_host(b747_handle* h, const void* act, void* obs, void* 
     CU(cudaEventCreateWithFlags(&b, cudaEventDisableTiming));
     h->ev_in.push_back(a); h->ev_k.push_back(b);
   }
+  return B747_OK;
+}
+
+// A copy between a caller's host buffer and its device staging: unit_bytes per envs_per_unit envs (1 for per-env
+// arrays, 32 for done bits; chunks start at whole thread blocks, so at whole units).
+struct HostXfer {
+  void* host;
+  void* dev;
+  size_t unit_bytes, envs_per_unit;
+  size_t off(size_t lo) const { return lo / envs_per_unit * unit_bytes; }
+  size_t len(size_t lo, size_t hi) const { return (hi - lo + envs_per_unit - 1) / envs_per_unit * unit_bytes; }
+};
+
+// Enqueue one env step with HOST buffers (b747_step_host, and b747_step_host_packed in copy mode): per chunk [lo, hi)
+// the copy-in, launch(lo, hi, stream) and the copy-outs in list order.  One chunk runs on `origin` alone.  More chunks
+// run as a pipeline -- actions of chunk c+1 go up and results of chunk c-1 come down (PCIe is full duplex, the copy
+// engines run beside the SMs) while chunk c is stepped; chunks alternate between two compute streams so that the tail
+// wave of one overlaps the head of the next.  The pipeline forks from `origin` and joins back into it, so the whole step
+// is ordered like a single operation on that stream -- and can be stream-captured.  Environments are independent, so
+// chunking cannot change any result.
+template <class Launch>
+static int issue_pipeline(b747_handle* h, cudaStream_t origin, const HostXfer& in, const HostXfer* outs, int n_outs,
+                          int chunks, size_t per, Launch launch) {
+  const size_t n = (size_t)h->cfg.n_envs;
+  const bool fork = chunks > 1;
+  const cudaStream_t s_in = fork ? h->s_in : origin, s_out = fork ? h->s_out : origin;
+  if (fork) {  // everything queued on the origin stream so far (resets, device-side steps) comes first
+    CU(cudaEventRecord(h->ev_start, origin));
+    CU(cudaStreamWaitEvent(h->s_in, h->ev_start, 0));
+    CU(cudaStreamWaitEvent(h->s_aux, h->ev_start, 0));
+  }
+  for (int c = 0; c < chunks; c++) {
+    const size_t lo = (size_t)c * per, hi = std::min(n, lo + per);
+    CU(cudaMemcpyAsync((char*)in.dev + in.off(lo), (char*)in.host + in.off(lo), in.len(lo, hi), cudaMemcpyHostToDevice, s_in));
+    const cudaStream_t sc = (c & 1) ? h->s_aux : origin;
+    if (fork) {
+      CU(cudaEventRecord(h->ev_in[c], s_in));
+      CU(cudaStreamWaitEvent(sc, h->ev_in[c], 0));
+    }
+    launch((int)lo, (int)hi, sc);
+    CU(cudaGetLastError());
+    if (fork) {
+      CU(cudaEventRecord(h->ev_k[c], sc));
+      CU(cudaStreamWaitEvent(s_out, h->ev_k[c], 0));
+    }
+    for (const HostXfer* o = outs; o < outs + n_outs; o++)
+      CU(cudaMemcpyAsync((char*)o->host + o->off(lo), (char*)o->dev + o->off(lo), o->len(lo, hi), cudaMemcpyDeviceToHost, s_out));
+  }
+  if (fork) {  // join: the copy-out stream has seen every chunk's kernel (and through them every copy-in)
+    CU(cudaEventRecord(h->ev_done, s_out));
+    CU(cudaStreamWaitEvent(origin, h->ev_done, 0));
+  }
+  return B747_OK;
+}
+
+static bool is_pinned(const void* p) {
+  cudaPointerAttributes a;
+  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
+  return a.type == cudaMemoryTypeHost;
+}
+
+extern "C" int b747_step_host(b747_handle* h, const void* act, void* obs, void* rew, uint8_t* done, void* term) {
+  if (!h || !act || !obs || !rew || !done) return fail(B747_ERR_ARG, "null argument");
+  if (!h->cfg.env_layer) return fail(B747_ERR_STATE, "handle was created with env_layer=0; use b747_model_step");
+  CU(cudaSetDevice(h->cfg.device));
+  const size_t es = h->elem(), od = (size_t)h->dc.obs_dim;
+  size_t per;
+  const int chunks = plan_chunks(h, true, per);
+  int rc = pipeline_resources(h, chunks);
+  if (rc != B747_OK) return rc;
+  const HostXfer in{(void*)act, h->d_act, es, 1};
+  const HostXfer outs[4] = {{obs, h->d_obs, es * od, 1}, {rew, h->d_rew, es, 1}, {done, h->d_done, 1, 1},
+                            {term, h->d_term, es * od, 1}};
+  const int n_outs = term ? 4 : 3;
+  void* d_term = term ? h->d_term : nullptr;
+  auto launch = [&](int lo, int hi, cudaStream_t s) { step_range(h, lo, hi, h->d_act, h->d_obs, h->d_rew, h->d_done, d_term, s); };
   // Pinned buffers: the ~70 stream operations of the pipeline are captured once per buffer set into a CUDA graph and
   // replayed with one launch call per step (the host-side issue time of the eager form is a third of the step).
-  if (h->use_graphs && is_pinned(act) && is_pinned(obs) && is_pinned(rew) && is_pinned(done) && (!term || is_pinned(term))) {
+  if (chunks > 1 && h->use_graphs && is_pinned(act) && is_pinned(obs) && is_pinned(rew) && is_pinned(done) &&
+      (!term || is_pinned(term))) {
     cudaGraphExec_t exec = nullptr;
     for (auto& g : h->graphs)
       if (g.act == act && g.obs == obs && g.rew == rew && g.done == done && g.term == term && g.chunks == chunks &&
@@ -501,7 +526,7 @@ extern "C" int b747_step_host(b747_handle* h, const void* act, void* obs, void* 
       // captured on an internal stream (the handle's stream may be the legacy default stream, which cannot capture)
       CU(cudaStreamBeginCapture(h->s_cap, cudaStreamCaptureModeThreadLocal));
       const int64_t launches0 = h->launches;
-      const int rc = issue_pipeline(h, h->s_cap, act, obs, rew, done, term, chunks, per);
+      rc = issue_pipeline(h, h->s_cap, in, outs, n_outs, chunks, per, launch);
       h->launches = launches0;
       const cudaError_t ce = cudaStreamEndCapture(h->s_cap, &graph);
       if (rc != B747_OK || ce != cudaSuccess || !graph) {
@@ -525,7 +550,7 @@ extern "C" int b747_step_host(b747_handle* h, const void* act, void* obs, void* 
       return B747_OK;
     }
   }
-  const int rc = issue_pipeline(h, h->stream, act, obs, rew, done, term, chunks, per);
+  rc = issue_pipeline(h, h->stream, in, outs, n_outs, chunks, per, launch);
   if (rc != B747_OK) return rc;
   CU(cudaStreamSynchronize(h->stream));
   return B747_OK;
@@ -562,26 +587,26 @@ extern "C" int b747_set_host_mode(b747_handle* h, int mode) {
   return B747_OK;
 }
 
-// device alias of a pinned (mapped) host pointer; nullptr if the memory is not device-accessible
-static void* mapped_ptr(const void* p) {
-  if (!is_pinned(p)) return nullptr;
+// device alias of a pinned (mapped) host pointer; nullptr if the memory is not pinned or not device-accessible
+static void* mapped_ptr(const void* p, bool pinned) {
   void* d = nullptr;
-  if (cudaHostGetDevicePointer(&d, (void*)p, 0) != cudaSuccess) { cudaGetLastError(); return nullptr; }
+  if (pinned && cudaHostGetDevicePointer(&d, (void*)p, 0) != cudaSuccess) { cudaGetLastError(); return nullptr; }
   return d;
 }
 
 extern "C" int b747_step_host_packed(b747_handle* h, const float* act, float* out4, uint32_t* done_bits) {
   if (!h || !act || !out4 || !done_bits) return fail(B747_ERR_ARG, "null argument");
-  const int prc = packed_ok(h);
-  if (prc) return prc;
+  int rc = packed_ok(h);
+  if (rc) return rc;
   CU(cudaSetDevice(h->cfg.device));
   const size_t n = (size_t)h->cfg.n_envs, np = (size_t)h->dc.n_pad, nw = (n + 31) / 32;
   const size_t rec4 = ((size_t)h->dc.obs_dim + 4) / 4;  // float4s per record
   if (!h->d_bits) CU(cudaMalloc(&h->d_bits, sizeof(uint32_t) * (np / 32)));
-  float* m_act = (float*)mapped_ptr(act);
-  float4* m_out = (float4*)mapped_ptr(out4);
+  const bool pin_act = is_pinned(act), pin_out = is_pinned(out4), pin_bits = is_pinned(done_bits);
+  float* m_act = (float*)mapped_ptr(act, pin_act);
+  float4* m_out = (float4*)mapped_ptr(out4, pin_out);
   int mode = h->host_mode;
-  const bool can_map = m_out && m_act && is_pinned(done_bits);
+  const bool can_map = m_out && m_act && pin_bits;
   bool calibrating = false;
   if (mode < 0) {
     mode = 2;
@@ -590,7 +615,7 @@ extern "C" int b747_step_host_packed(b747_handle* h, const float* act, float* ou
       else { calibrating = true; mode = (h->auto_calls & 1) ? 0 : 2; }
     }
   }
-  if (!m_out || !is_pinned(done_bits)) mode = 0;
+  if (!m_out || !pin_bits) mode = 0;
   if (mode == 2 && !m_act) mode = 1;
   const auto t_begin = std::chrono::steady_clock::now();
   struct Calib {  // on every return path: book the call's time and decide after 4 + 4 calls (the first pair is warm-up)
@@ -619,58 +644,22 @@ extern "C" int b747_step_host_packed(b747_handle* h, const float* act, float* ou
     CU(cudaStreamSynchronize(h->stream));
     return B747_OK;
   }
-  // copy mode (pageable buffers, or asked for): H2D, step into device staging, D2H -- chunked like b747_step_host when
-  // the buffers are pinned
+  // copy mode (pageable buffers, or asked for): the host-step pipeline of b747_step_host with records and done words;
+  // chunked only when all three buffers are pinned
   if (!h->d_out4) CU(cudaMalloc(&h->d_out4, sizeof(float4) * rec4 * np));
-  const bool pinned = is_pinned(act) && is_pinned(out4) && is_pinned(done_bits);
-  int chunks = (pinned && n >= ((size_t)1 << 17)) ? (h->host_chunks ? h->host_chunks : 4) : 1;
-  const size_t per = ((n + chunks - 1) / chunks + 127) / 128 * 128;
-  chunks = (int)((n + per - 1) / per);
-  if (chunks > 1) {
-    if (!h->s_in) {
-      CU(cudaStreamCreateWithFlags(&h->s_in, cudaStreamNonBlocking));
-      CU(cudaStreamCreateWithFlags(&h->s_aux, cudaStreamNonBlocking));
-      CU(cudaStreamCreateWithFlags(&h->s_out, cudaStreamNonBlocking));
-      CU(cudaStreamCreateWithFlags(&h->s_cap, cudaStreamNonBlocking));
-      CU(cudaEventCreateWithFlags(&h->ev_start, cudaEventDisableTiming));
-      CU(cudaEventCreateWithFlags(&h->ev_done, cudaEventDisableTiming));
-    }
-    while ((int)h->ev_in.size() < chunks) {
-      cudaEvent_t a, b;
-      CU(cudaEventCreateWithFlags(&a, cudaEventDisableTiming));
-      CU(cudaEventCreateWithFlags(&b, cudaEventDisableTiming));
-      h->ev_in.push_back(a); h->ev_k.push_back(b);
-    }
-    CU(cudaEventRecord(h->ev_start, h->stream));
-    CU(cudaStreamWaitEvent(h->s_in, h->ev_start, 0));
-    CU(cudaStreamWaitEvent(h->s_aux, h->ev_start, 0));
-    for (int c = 0; c < chunks; c++) {
-      const size_t lo = (size_t)c * per, hi = std::min(n, lo + per), m = hi - lo;
-      CU(cudaMemcpyAsync((float*)h->d_act + lo, act + lo, sizeof(float) * m, cudaMemcpyHostToDevice, h->s_in));
-      CU(cudaEventRecord(h->ev_in[c], h->s_in));
-      cudaStream_t sc = (c & 1) ? h->s_aux : h->stream;
-      CU(cudaStreamWaitEvent(sc, h->ev_in[c], 0));
-      DevCfg dc = h->dc;
-      dc.env_lo = (int)lo; dc.env_hi = (int)hi;
-      launch_env_step32(dc, h->s32, (const float*)h->d_act, nullptr, nullptr, nullptr, nullptr, sc, h->d_out4, h->d_bits);
-      h->launches++;
-      CU(cudaGetLastError());
-      CU(cudaEventRecord(h->ev_k[c], sc));
-      CU(cudaStreamWaitEvent(h->s_out, h->ev_k[c], 0));
-      CU(cudaMemcpyAsync(out4 + 4 * rec4 * lo, h->d_out4 + rec4 * lo, sizeof(float4) * rec4 * m, cudaMemcpyDeviceToHost, h->s_out));
-      CU(cudaMemcpyAsync(done_bits + lo / 32, h->d_bits + lo / 32, sizeof(uint32_t) * ((m + 31) / 32), cudaMemcpyDeviceToHost, h->s_out));
-    }
-    CU(cudaEventRecord(h->ev_done, h->s_out));
-    CU(cudaStreamWaitEvent(h->stream, h->ev_done, 0));
-    CU(cudaStreamSynchronize(h->stream));
-    return B747_OK;
-  }
-  CU(cudaMemcpyAsync(h->d_act, act, sizeof(float) * n, cudaMemcpyHostToDevice, h->stream));
-  launch_env_step32(h->dc, h->s32, (const float*)h->d_act, nullptr, nullptr, nullptr, nullptr, h->stream, h->d_out4, h->d_bits);
-  h->launches++;
-  CU(cudaGetLastError());
-  CU(cudaMemcpyAsync(out4, h->d_out4, sizeof(float4) * rec4 * n, cudaMemcpyDeviceToHost, h->stream));
-  CU(cudaMemcpyAsync(done_bits, h->d_bits, sizeof(uint32_t) * nw, cudaMemcpyDeviceToHost, h->stream));
+  size_t per;
+  const int chunks = plan_chunks(h, pin_act && pin_out && pin_bits, per);
+  rc = pipeline_resources(h, chunks);
+  if (rc != B747_OK) return rc;
+  const HostXfer in{(void*)act, h->d_act, sizeof(float), 1};
+  const HostXfer outs[2] = {{out4, h->d_out4, sizeof(float4) * rec4, 1}, {done_bits, h->d_bits, sizeof(uint32_t), 32}};
+  rc = issue_pipeline(h, h->stream, in, outs, 2, chunks, per, [&](int lo, int hi, cudaStream_t s) {
+    DevCfg dc = h->dc;
+    dc.env_lo = lo; dc.env_hi = hi;
+    launch_env_step32(dc, h->s32, (const float*)h->d_act, nullptr, nullptr, nullptr, nullptr, s, h->d_out4, h->d_bits);
+    h->launches++;
+  });
+  if (rc != B747_OK) return rc;
   CU(cudaStreamSynchronize(h->stream));
   return B747_OK;
 }

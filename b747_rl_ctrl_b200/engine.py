@@ -188,7 +188,8 @@ class BatchEngine:
         self.cfg.seed = int(seed) & (2 ** 64 - 1)
 
     def set_host_chunks(self, n_chunks):
-        """Chunks of step_host's copy/compute pipeline: 0 = automatic, 1 = one launch."""
+        """Chunks of the copy/compute pipeline of step_host and of step_host_packed's staged copies (mode 0, pinned
+        buffers): 0 = automatic, 1 = one launch."""
         check(self._L.b747_set_host_chunks(self._h, int(n_chunks)))
 
     def model_step(self, n_steps=1):

@@ -126,7 +126,8 @@ int b747_step(b747_handle *h, const void *actions_dev, void *obs_dev, void *rew_
  * pipelined over env chunks (copy-in, step and copy-out of neighbouring chunks overlap; pinned buffers
  * are needed for the overlap, pageable ones still work); results are identical to the one-launch form. */
 int b747_step_host(b747_handle *h, const void *actions, void *obs, void *rew, uint8_t *done, void *terminal_obs);
-/* Number of chunks of b747_step_host's pipeline: 0 = automatic (4 from 128 Ki envs, else 1), 1 = no pipeline. */
+/* Number of chunks of the host-step pipeline of b747_step_host and of b747_step_host_packed's staged copies (mode 0,
+ * pinned buffers): 0 = automatic (4 from 128 Ki envs, else 1), 1 = no pipeline. */
 int b747_set_host_chunks(b747_handle *h, int n_chunks);
 
 /* Packed outputs (f32 handles): per env ONE record of R = b747_packed_record_floats(obs_type) = 4 * ceil((obs_dim + 1) / 4)
@@ -144,10 +145,11 @@ int b747_set_host_chunks(b747_handle *h, int n_chunks);
 int b747_packed_record_floats(int obs_type);
 int b747_step_packed(b747_handle *h, const float *actions_dev, float *out4_dev, uint32_t *done_bits_dev);
 int b747_step_host_packed(b747_handle *h, const float *actions, float *out4, uint32_t *done_bits);
-/* Host path of b747_step_host_packed with page-locked buffers: 0 staged copies (chunk pipeline), 1 actions copied /
- * records stored zero-copy, 2 actions and records zero-copy, -1 automatic (default): the first ten calls alternate
- * between 2 and 0 and are timed, the faster path is kept (zero-copy when the GPU has the host link to itself, staged
- * copies when many GPUs share it).  Results are identical in every mode. */
+/* Host path of b747_step_host_packed with page-locked buffers: 0 staged copies (the chunk pipeline of b747_step_host;
+ * b747_set_host_chunks applies), 1 actions copied / records stored zero-copy, 2 actions and records zero-copy,
+ * -1 automatic (default): the first ten calls alternate between 2 and 0 and are timed, the faster path is kept
+ * (zero-copy when the GPU has the host link to itself, staged copies when many GPUs share it).  Results are identical
+ * in every mode. */
 int b747_set_host_mode(b747_handle *h, int mode);
 /* env.seed(s) of the gym / SB3 API (neural/agent.py:80): re-keys the Philox stream used by every later random reset. */
 int b747_set_seed(b747_handle *h, uint64_t seed);

@@ -166,10 +166,12 @@ def test_vec_env_contract(oracle):
     venv.close()
 
 
-@pytest.mark.parametrize("n,mode", [(1000, -1), (1000, 0), (1000, 1), (200000, -1), (200000, 0), (777, "pageable")])
+@pytest.mark.parametrize("n,mode", [(1000, -1), (1000, 0), (1000, 1), (200000, -1), (200000, 0), (777, "pageable"),
+                                    (5000, "chunked")])
 def test_packed_host_step_equals_plain_step(n, mode):
     """b747_step_host_packed (one float4 record per env + done bits; zero-copy on pinned buffers, staged copies
-    otherwise) returns exactly what b747_step_host returns: record = (terminal observation, reward), bit = done."""
+    otherwise) returns exactly what b747_step_host returns: record = (terminal observation, reward), bit = done.
+    "chunked": staged copies (mode 0) pipelined over set_host_chunks(7) chunks, below the automatic chunking's size."""
     import torch
     from b747_rl_ctrl_b200 import engine as E
     kw = dict(dtype=E.F32, seed=6, sample_time=0.05, tk=0.35)  # 7-step episodes: auto-resets inside the run
@@ -179,7 +181,9 @@ def test_packed_host_step_equals_plain_step(n, mode):
     if mode == "pageable":
         act, out4, bits = np.zeros(n, np.float32), np.zeros((n, 4), np.float32), np.zeros(nw, np.uint32)
     else:
-        pk.set_host_mode(mode)
+        if mode == "chunked":
+            pk.set_host_chunks(7)
+        pk.set_host_mode(0 if mode == "chunked" else mode)
         keep = [torch.zeros(n).pin_memory(), torch.zeros(n, 4).pin_memory(), torch.zeros(nw, dtype=torch.int32).pin_memory()]
         act, out4, bits = keep[0].numpy(), keep[1].numpy(), keep[2].numpy().view(np.uint32)
     rng = np.random.default_rng(2)
@@ -197,6 +201,9 @@ def test_packed_host_step_equals_plain_step(n, mode):
         assert np.array_equal(out4[:, :3], term) and np.array_equal(out4[:, 3], rew), k
         n_done += int(done.sum())
     assert n_done == 2 * n
+    if mode == "chunked":
+        per = -(-(-(-n // 7)) // 128) * 128  # whole thread blocks per chunk
+        assert pk.launch_count - ref.launch_count == 16 * (-(-n // per) - 1)
     s0, s1 = ref.episode_stats(), pk.episode_stats()
     assert s0[0] == s1[0] == 2 * n and np.allclose(s0, s1, rtol=1e-12)
     for name in ("h", "th", "tick", "ep_idx", "ep_return"):
