@@ -94,6 +94,10 @@ def load():
     L.b747_episode_stats.argtypes = [vp, c_dp]
     L.b747_last_episode.argtypes = [vp, vp, vp]
     L.b747_last_episode_of.argtypes = [vp, vp, ctypes.c_int32, vp, vp]
+    L.b747_state_bytes.restype = ctypes.c_int64
+    L.b747_state_bytes.argtypes = [ctypes.POINTER(Cfg), ctypes.c_int32]
+    L.b747_save_state.argtypes = [vp, vp, ctypes.c_int32, vp]
+    L.b747_load_state.argtypes = [vp, vp, vp, vp, ctypes.c_int32]
     L.b747_launch_count.restype = ctypes.c_int64
     L.b747_launch_count.argtypes = [vp]
     L.b747_synchronize.argtypes = [vp]

@@ -25,6 +25,7 @@ UNITS = {
     # throughput kernels: approximate (1-2 ulp) float32 division / sqrt; float64 ops unaffected
     "b747_kernels_f32.cu": ["-prec-div=false", "-prec-sqrt=false"],
     "b747_capi.cu": [],
+    "b747_state.cu": [],
     "b747_scalar.cu": [],
     "b747_scalar_legacy.cu": [],
 }
@@ -62,7 +63,7 @@ def build_native(force=False, verbose=False):
             if verbose:
                 print(" ".join(cmd))
             subprocess.run(cmd, check=True)
-    core = [objs[k] for k in ("b747_kernels_f64.cu", "b747_kernels_f32.cu", "b747_capi.cu")]
+    core = [objs[k] for k in ("b747_kernels_f64.cu", "b747_kernels_f32.cu", "b747_capi.cu", "b747_state.cu")]
     lib = os.path.join(LIBDIR, "libb747_b200.so")
     if force or _stale(lib, core):
         subprocess.run([nvcc] + ARCH + ["-shared", "-o", lib] + core + ["-Xlinker", "-Bsymbolic", "-lcudart_static", "-lpthread", "-ldl", "-lrt"],

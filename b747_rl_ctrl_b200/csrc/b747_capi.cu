@@ -778,6 +778,61 @@ extern "C" int b747_set_field(b747_handle* h, int field, const double* in) {
   return field_io(h, field, nullptr, in);
 }
 
+// ---- state save / load (row table and copy kernel in b747_state.cu) -----------------------------------
+static bool dtype_ok(int dtype) { return dtype == B747_F64 || dtype == B747_F32; }
+
+extern "C" int64_t b747_state_bytes(const b747_cfg* cfg, int32_t n) {
+  if (!cfg || n < 0 || !dtype_ok(cfg->dtype)) return fail(B747_ERR_ARG, "bad argument");
+  return (int64_t)state_blob_bytes(state_table(*cfg, 0, nullptr, nullptr, nullptr), n);
+}
+
+static StateTable handle_state(const b747_handle* h) {
+  return state_table(h->cfg, (size_t)h->dc.n_pad, &h->s32, &h->s64, &h->trace);
+}
+
+// the copy kernel moves 16-byte rows with 128-bit accesses at 16-byte offsets from the blob and reads int32 indices: a
+// misaligned pointer would fault the context, so it is refused before anything is launched
+static int state_ptrs_ok(const void* blob, const int32_t* a, const int32_t* b) {
+  if ((uintptr_t)blob & 15) return fail(B747_ERR_ARG, "state blob must be 16-byte aligned");
+  if (((uintptr_t)a | (uintptr_t)b) & 3) return fail(B747_ERR_ARG, "index arrays must be 4-byte aligned");
+  return B747_OK;
+}
+
+extern "C" int b747_save_state(b747_handle* h, const int32_t* env_idx, int32_t n, void* blob) {
+  if (!h || !blob || n < 0) return fail(B747_ERR_ARG, "bad argument");
+  if (!env_idx && n > h->cfg.n_envs) return fail(B747_ERR_ARG, "n > n_envs without an index array");
+  if (const int rc = state_ptrs_ok(blob, env_idx, nullptr)) return rc;
+  CU(cudaSetDevice(h->cfg.device));
+  const StateHeader hd = state_header(h->cfg, n, h->dc.force_full != 0);
+  launch_state_copy(handle_state(h), (char*)blob, n, env_idx, nullptr, n, h->cfg.n_envs, true, hd, h->stream);
+  h->launches++;
+  CU(cudaGetLastError());
+  return B747_OK;
+}
+
+extern "C" int b747_load_state(b747_handle* h, const void* blob, const int32_t* blob_idx, const int32_t* env_idx,
+                               int32_t n) {
+  if (!h || !blob || n < 0) return fail(B747_ERR_ARG, "bad argument");
+  if (!env_idx && n > h->cfg.n_envs) return fail(B747_ERR_ARG, "n > n_envs without an index array");
+  if (const int rc = state_ptrs_ok(blob, env_idx, blob_idx)) return rc;
+  CU(cudaSetDevice(h->cfg.device));
+  StateHeader hd;
+  CU(cudaMemcpyAsync(&hd, blob, sizeof hd, cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  const StateHeader want = state_header(h->cfg, hd.n, false);
+  if (hd.magic != want.magic || hd.version != want.version || hd.n < 0)
+    return fail(B747_ERR_STATE, "not a state blob of this format version");
+  if (hd.dtype != want.dtype) return fail(B747_ERR_STATE, "state blob was saved from a handle of the other dtype");
+  if (hd.key != want.key) return fail(B747_ERR_STATE, "state blob was saved from a handle with another configuration");
+  // a restored closed altitude loop (or oscillating reference, aero errors) needs the full f32 kernel tier
+  if ((hd.flags & kStateForceFull) && !h->dc.force_full) { h->dc.force_full = 1; h->epoch++; }
+  launch_state_copy(handle_state(h), (char*)blob, hd.n, env_idx, blob_idx, n, h->cfg.n_envs, false, hd, h->stream);
+  h->launches++;
+  CU(cudaGetLastError());
+  CU(cudaStreamSynchronize(h->stream));
+  return B747_OK;
+}
+
 // ---- episode statistics -----------------------------------------------------------------------
 extern "C" int b747_episode_stats(b747_handle* h, double out[4]) {
   if (!h || !out) return fail(B747_ERR_ARG, "null argument");

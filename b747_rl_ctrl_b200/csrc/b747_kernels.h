@@ -34,8 +34,52 @@ struct StateF32 {
   unsigned int* tile_ctr = nullptr;  // 64 tile counters of the persistent step kernel (one per launch in flight)
 };
 
+// A handle's per-env storage as row blocks for b747_save_state / b747_load_state: n_rows rows of elem bytes per env
+// (4, 8 or 16), row r of env i at base + r * stride + i * elem.  The blob stores each row as its entries padded to
+// 16 bytes (state_blob_bytes); a table built without a handle (null bases) still gives every size.
+struct StateBlock {
+  char* base;
+  size_t stride;  // bytes between rows
+  int32_t elem, n_rows;
+};
+constexpr int kMaxStateBlocks = 12;
+struct StateTable {
+  StateBlock b[kMaxStateBlocks];
+  int n_blocks = 0, n_rows = 0;
+  void add(const void* base, int elem, size_t stride, int n_rows_) {
+    b[n_blocks++] = {(char*)base, stride, elem, n_rows_};
+    n_rows += n_rows_;
+  }
+};
+// Leading 64 bytes of a blob.  key: hash of every b747_cfg field that fixes the layout or meaning of the state
+// (all but n_envs, device, seed, env_id_offset).
+struct StateHeader {
+  uint32_t magic, version;
+  int32_t dtype, n;
+  uint32_t flags;  // kStateForceFull
+  uint32_t reserved0;
+  uint64_t key;
+  uint64_t reserved[4];
+};
+static_assert(sizeof(StateHeader) == 64, "blob rows start 16-byte aligned");
+constexpr uint32_t kStateMagic = 0x53373437u;  // "747S"
+constexpr uint32_t kStateVersion = 1;
+constexpr uint32_t kStateForceFull = 1;        // the saving handle ran the full f32 kernel tier (DevCfg::force_full)
+
+// np: the handle's n_pad; s32 / s64 / trace may be null (sizes only).
+StateTable state_table(const b747_cfg& cfg, size_t np, const StateF32* s32, const StateF64* s64,
+                       const TraceState* trace);
+size_t state_blob_bytes(const StateTable& t, int n);
+StateHeader state_header(const b747_cfg& cfg, int n, bool force_full);
+// save: blob entry k <- env env_idx[k] (+ the header); load: env env_idx[k] <- blob entry blob_idx[k] of a blob of
+// blob_n entries.  Null index arrays are the identity; out-of-range entries skip k.
+void launch_state_copy(const StateTable& t, char* blob, int blob_n, const int32_t* env_idx, const int32_t* blob_idx,
+                       int n, int n_envs, bool save, const StateHeader& hdr, cudaStream_t s);
+
 int f32_alloc(const DevCfg& c, StateF32& s, bool export_signals, cudaStream_t stream);
 void f32_free(StateF32& s);
+// the row blocks of what f32_alloc allocates per env (s may be null)
+void f32_state_blocks(size_t np, bool export_signals, const StateF32* s, StateTable& t);
 bool f32_is_lean(const DevCfg& c);
 bool f32_needs_cs(const DevCfg& c);
 void f32_warm_launch();

@@ -584,6 +584,14 @@ int f32_alloc(const DevCfg& c, StateF32& s, bool export_signals, cudaStream_t st
   return 0;
 }
 
+void f32_state_blocks(size_t np, bool export_signals, const StateF32* s, StateTable& t) {
+  t.add(s ? s->D : nullptr, sizeof(double2), sizeof(double2) * np, ND_GROUPS);
+  t.add(s ? s->F : nullptr, sizeof(float4), sizeof(float4) * np, NF_GROUPS);
+  t.add(s ? s->last_ret : nullptr, sizeof(double), 0, 1);
+  t.add(s ? s->last_len : nullptr, sizeof(int), 0, 1);
+  if (export_signals) t.add(s ? s->sig : nullptr, sizeof(float), sizeof(float) * np, NSIG);
+}
+
 void f32_free(StateF32& s) {
   cudaFree(s.D); cudaFree(s.F); cudaFree(s.sig); cudaFree(s.stats); cudaFree(s.last_ret); cudaFree(s.last_len); cudaFree(s.tables); cudaFree(s.tile_ctr);
   s = StateF32{};

@@ -249,6 +249,93 @@ class BatchEngine:
         check(self._L.b747_recorder_read(self._h, int(env), _ptr(buf), ctypes.byref(n)))
         return {nm: buf[k, :n.value].copy() for k, nm in enumerate(names)}
 
+    # -- state save / load (checkpoint, resume, fork) --------------------------------------------------------
+    def state_bytes(self, n=None):
+        """Bytes of a state blob holding n envs (default: all) of this handle's configuration."""
+        b = int(self._L.b747_state_bytes(ctypes.byref(self.cfg), self.n_envs if n is None else int(n)))
+        if b < 0:
+            check(b)
+        return b
+
+    def _device(self):
+        return self._th().device("cuda", self.cfg.device)
+
+    def _dev_index(self, idx):
+        """Contiguous int32 device tensor of an index list (numpy array, sequence or tensor); None stays None."""
+        if idx is None:
+            return None
+        th = self._th()
+        t = idx if isinstance(idx, th.Tensor) else th.from_numpy(np.ascontiguousarray(idx, np.int32).reshape(-1))
+        return t.to(device=self._device(), dtype=th.int32).contiguous().reshape(-1)
+
+    def _order(self, after_torch):
+        """after_torch: the handle's stream waits for what torch's current stream queued so far (index and blob
+        tensors); else torch's current stream waits for the handle's."""
+        th = self._th()
+        dev = self._device()
+        handle = th.cuda.ExternalStream(self.stream_ptr or 0, device=dev)
+        cur = th.cuda.current_stream(dev)
+        src, dst = (cur, handle) if after_torch else (handle, cur)
+        ev = th.cuda.Event()
+        ev.record(src)
+        dst.wait_event(ev)
+
+    def save_state(self, indices=None, out=None):
+        """State blob (torch.uint8 device tensor) of the envs `indices` (numpy array or int32 device tensor; default
+        every env in order): entry k holds env indices[k].  `out`: a preallocated uint8 device tensor of at least
+        state_bytes(n) bytes.  Asynchronous; torch's current stream is ordered after the copy.  A checkpoint on disk
+        is the blob's .cpu() copy."""
+        th = self._th()
+        idx = self._dev_index(indices)
+        n = self.n_envs if idx is None else idx.numel()
+        nb = self.state_bytes(n)
+        if out is None:
+            out = th.empty(nb, dtype=th.uint8, device=self._device())
+        elif (out.dtype != th.uint8 or out.device != self._device() or not out.is_contiguous() or out.numel() < nb
+              or out.data_ptr() % 16):
+            raise ValueError(f"out must be a contiguous, 16-byte aligned uint8 tensor of at least {nb} bytes on "
+                             f"{self._device()}")
+        self._order(after_torch=True)
+        check(self._L.b747_save_state(self._h, _ptr(idx), n, _ptr(out)))
+        self._order(after_torch=False)
+        return out
+
+    def load_state(self, blob, indices=None, blob_indices=None):
+        """Env indices[k] <- blob entry blob_indices[k] (either None: the identity; both None: every env from the entry
+        of the same number).  blob: what save_state returned, on this device, another one or the host (copied here,
+        and to a fresh tensor where it does not start 16-byte aligned).  Raises B747Error if the blob is not a state
+        blob of this handle's dtype and configuration, ValueError if it is shorter than its header says.
+        Synchronised."""
+        th = self._th()
+        b = blob if isinstance(blob, th.Tensor) else th.from_numpy(np.ascontiguousarray(blob).reshape(-1).view(np.uint8))
+        if b.dtype != th.uint8 or b.dim() != 1:
+            raise ValueError("blob must be a 1-D uint8 tensor (BatchEngine.save_state)")
+        if b.numel() < 64:
+            raise B747Error("not a state blob: shorter than its 64-byte header")
+        head = b[:64].cpu().numpy()
+        # magic, version, dtype (bytes 0-11) and configuration key (24-31) against a 0-env blob of this handle, so that a
+        # foreign blob is refused like the C call refuses it before its size is judged by this handle's layout
+        own = th.empty(64, dtype=th.uint8, device=self._device())
+        self._order(after_torch=True)
+        check(self._L.b747_save_state(self._h, None, 0, _ptr(own)))
+        self._order(after_torch=False)
+        own = own.cpu().numpy()
+        if not (np.array_equal(head[:12], own[:12]) and np.array_equal(head[24:32], own[24:32])):
+            raise B747Error("not a state blob of this handle's dtype and configuration (magic, version, dtype or key "
+                            "differ)")
+        n_blob = int(head[12:16].view(np.int32)[0])
+        if n_blob < 0 or b.numel() < self.state_bytes(n_blob):
+            raise ValueError(f"blob is shorter than a blob of its {n_blob} entries: truncated")
+        b = b.to(self._device()).contiguous()
+        if b.data_ptr() % 16:
+            b = b.clone()   # fresh allocations are aligned
+        idx, bidx = self._dev_index(indices), self._dev_index(blob_indices)
+        if idx is not None and bidx is not None and idx.numel() != bidx.numel():
+            raise ValueError("indices and blob_indices differ in length")
+        n = idx.numel() if idx is not None else (bidx.numel() if bidx is not None else self.n_envs)
+        self._order(after_torch=True)
+        check(self._L.b747_load_state(self._h, _ptr(b), _ptr(bidx), _ptr(idx), n))
+
     # -- episode statistics ---------------------------------------------------------------------
     def episode_stats(self):
         """(episodes finished, sum of returns, sum of lengths, sum of squared returns) since the last call."""

@@ -520,6 +520,36 @@ class B747VecEnv(_VecEnvBase):
         """(episodes, sum of returns, sum of lengths, sum of squared returns) since the last call."""
         return self.engine.episode_stats()
 
+    # ---- checkpoint / resume ----------------------------------------------------------------------------
+    def get_state(self):
+        """Checkpoint of every env: {"engine": the handle's state blob (BatchEngine.save_state, a device tensor),
+        "obs", "rew": copies of what the last reset or step returned (None before the first reset)}."""
+        obs, rew = self._last if self._last is not None else (None, None)
+        cp = lambda x: None if x is None else (x.clone() if hasattr(x, "clone") else np.array(x, copy=True))
+        return {"engine": self.engine.save_state(), "obs": cp(obs), "rew": cp(rew)}
+
+    def set_state(self, state):
+        """Restore a get_state() checkpoint of an env created with the same arguments; returns the observation to
+        continue from (SB3's `_last_obs`), as reset() would."""
+        self.engine.load_state(state["engine"])
+        self._clean_infos()
+        od, dt = self.engine.obs_dim, self.engine.np_dtype
+        obs, rew = state["obs"], state["rew"]
+        if self.device_tensors:
+            if obs is None:
+                self._obs_d.zero_()
+                self._rew_d.zero_()
+            else:
+                self._obs_d.copy_(obs)
+                self._rew_d.copy_(rew)
+            self._last = (self._obs_d, self._rew_d)
+            return self._obs_d
+        host = lambda x: np.array(x.cpu().numpy() if hasattr(x, "cpu") else x, dtype=dt, copy=True)
+        obs = np.zeros((self.num_envs, od), dt) if obs is None else host(obs)
+        rew = np.zeros(self.num_envs, dt) if rew is None else host(rew)
+        self._last = (obs, rew)
+        return obs.copy()
+
     @property
     def unwrapped(self):
         return self

@@ -200,6 +200,31 @@ int b747_recorder_n_fields(void);
 const char *b747_recorder_field_name(int field);
 int b747_recorder_read(b747_handle *h, int env, double *out_host, int32_t *n_steps);
 
+/* Save, restore and fork per-env state.  A state blob is device memory: a 64-byte header (magic, format version,
+ * dtype, n, flags, a 64-bit key of every b747_cfg field except n_envs, device, seed and env_id_offset) followed by n
+ * entries of every per-env array the handle allocates, byte for byte -- f32 handles: the double2 and float4 state
+ * groups (tick word with its look-up hints, episode index), last_ret, last_len; f64 handles: every slot including
+ * state0, tick, flags, ep_idx, last_ret, last_len; both: the exported signals, the transfer tracker and its snapshot,
+ * and the recorder rows when the handle has them.  Not in a blob: b747_set_param tunables, the seed, the
+ * b747_episode_stats accumulators and the handle's scratch.  After a load, later random resets of env j are drawn
+ * from the loading handle's seed, its env_id_offset + j and the episode index that came from the blob.
+ * The blob must be 16-byte aligned (cudaMalloc and torch allocations are; a slice at another offset is not), index
+ * arrays are int32 device arrays; a misaligned pointer is B747_ERR_ARG and nothing is launched.  An index entry outside
+ * [0, n_envs) or outside [0, blob n) skips that k (nothing is written).  Duplicate env_idx entries in a load give an
+ * unspecified result without a fault: that env's rows may come from different ones of its entries.
+ *
+ * b747_state_bytes: bytes of a blob holding n envs of a handle created with *cfg (no GPU needed); < 0 on a bad argument.
+ * b747_save_state: blob entry k <- env env_idx_dev[k] for k < n (env_idx_dev NULL: env k, n <= n_envs).
+ *   Asynchronous on the handle's stream.
+ * b747_load_state: env env_idx_dev[k] <- blob entry blob_idx_dev[k] for k < n (NULL: identity; env_idx_dev NULL needs
+ *   n <= n_envs).  Reads the header first and returns B747_ERR_STATE, writing nothing, on a wrong magic or version,
+ *   another dtype or another configuration key.  A blob saved by a handle that ran the full f32 kernel tier moves this
+ *   handle there too (like b747_reset_to with a closed altitude loop).  Synchronised on return. */
+int64_t b747_state_bytes(const b747_cfg *cfg, int32_t n);
+int b747_save_state(b747_handle *h, const int32_t *env_idx_dev, int32_t n, void *blob_dev);
+int b747_load_state(b747_handle *h, const void *blob_dev, const int32_t *blob_idx_dev, const int32_t *env_idx_dev,
+                    int32_t n);
+
 /* Number of kernel launches issued through this handle so far (bench.py's gpu_launches). */
 int64_t b747_launch_count(b747_handle *h);
 int b747_synchronize(b747_handle *h);
