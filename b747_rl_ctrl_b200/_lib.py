@@ -98,6 +98,9 @@ def load():
     L.b747_state_bytes.argtypes = [ctypes.POINTER(Cfg), ctypes.c_int32]
     L.b747_save_state.argtypes = [vp, vp, ctypes.c_int32, vp]
     L.b747_load_state.argtypes = [vp, vp, vp, vp, ctypes.c_int32]
+    L.b747_set_env_param.argtypes = [vp, ctypes.c_char_p, vp, vp, ctypes.c_int32]
+    L.b747_get_env_param.argtypes = [vp, ctypes.c_char_p, vp, ctypes.c_int32, vp]
+    L.b747_set_env_param_range.argtypes = [vp, ctypes.c_char_p, c_dp, c_dp, c_int]
     L.b747_launch_count.restype = ctypes.c_int64
     L.b747_launch_count.argtypes = [vp]
     L.b747_synchronize.argtypes = [vp]

@@ -55,8 +55,10 @@ struct b747_handle {
   b747_episode* d_eps = nullptr;
   double* d_metrics = nullptr;  // [n_pad][5] staging for b747_transfer_metrics
   TraceState trace;
+  EnvParams pe;  // per-env tunables: rows allocated by the first b747_set_env_param / b747_set_env_param_range
   int64_t launches = 0;
   size_t elem() const { return cfg.dtype == B747_F64 ? 8 : 4; }
+  const EnvParams* per_env() const { return pe.rows ? &pe : nullptr; }
 };
 
 extern "C" const char* b747_last_error(void) { return g_err.c_str(); }
@@ -278,6 +280,7 @@ extern "C" int b747_destroy(b747_handle* h) {
   cudaFree(s.slots); cudaFree(s.tick); cudaFree(s.flags); cudaFree(s.ep_idx); cudaFree(s.sig); cudaFree(s.stats);
   cudaFree(s.last_ret); cudaFree(s.last_len);
   f32_free(h->s32);
+  cudaFree(h->pe.rows); cudaFree(h->pe.phys); cudaFree(h->pe.ss);
   cudaFree(h->d_act); cudaFree(h->d_obs); cudaFree(h->d_rew); cudaFree(h->d_term); cudaFree(h->d_done); cudaFree(h->d_eps);
   if (h->own_stream && h->stream) cudaStreamDestroy(h->stream);
   for (cudaEvent_t e : h->ev_in) cudaEventDestroy(e);
@@ -351,9 +354,9 @@ extern "C" int b747_synchronize(b747_handle* h) {
 extern "C" int b747_reset(b747_handle* h, const uint8_t* mask_dev, void* obs_dev) {
   if (!h) return fail(B747_ERR_ARG, "null handle");
   CU(cudaSetDevice(h->cfg.device));
-  if (h->cfg.dtype == B747_F64) launch_reset64(h->dc, h->s64, mask_dev, nullptr, (double*)obs_dev, h->stream);
-  else launch_reset32(h->dc, h->s32, mask_dev, nullptr, (float*)obs_dev, h->stream);
-  h->launches++;
+  if (h->cfg.dtype == B747_F64) launch_reset64(h->dc, h->s64, mask_dev, nullptr, (double*)obs_dev, h->stream, h->per_env());
+  else launch_reset32(h->dc, h->s32, mask_dev, nullptr, (float*)obs_dev, h->stream, h->per_env());
+  h->launches += (h->pe.ranged && h->dc.reset_ref_mode != B747_RESET_NONE) ? 2 : 1;
   CU(cudaGetLastError());
   return B747_OK;
 }
@@ -388,9 +391,10 @@ static void step_range(b747_handle* h, int lo, int hi, const void* act, void* ob
   DevCfg dc = h->dc;
   dc.env_lo = lo; dc.env_hi = hi;
   if (h->cfg.dtype == B747_F64)
-    launch_env_step64(dc, h->s64, (const double*)act, (double*)obs, (double*)rew, done, (double*)term, s);
+    launch_env_step64(dc, h->s64, (const double*)act, (double*)obs, (double*)rew, done, (double*)term, s, h->per_env());
   else
-    launch_env_step32(dc, h->s32, (const float*)act, (float*)obs, (float*)rew, done, (float*)term, s);
+    launch_env_step32(dc, h->s32, (const float*)act, (float*)obs, (float*)rew, done, (float*)term, s, nullptr, nullptr,
+                      false, h->per_env());
   h->launches++;
 }
 
@@ -574,7 +578,8 @@ extern "C" int b747_step_packed(b747_handle* h, const float* act_dev, float* out
   const int rc = packed_ok(h);
   if (rc) return rc;
   CU(cudaSetDevice(h->cfg.device));
-  launch_env_step32(h->dc, h->s32, act_dev, nullptr, nullptr, nullptr, nullptr, h->stream, (float4*)out4_dev, done_bits_dev);
+  launch_env_step32(h->dc, h->s32, act_dev, nullptr, nullptr, nullptr, nullptr, h->stream, (float4*)out4_dev, done_bits_dev,
+                    false, h->per_env());
   h->launches++;
   CU(cudaGetLastError());
   return B747_OK;
@@ -637,7 +642,8 @@ extern "C" int b747_step_host_packed(b747_handle* h, const float* act, float* ou
       CU(cudaMemcpyAsync(h->d_act, act, sizeof(float) * n, cudaMemcpyHostToDevice, h->stream));
       a_dev = (const float*)h->d_act;
     }
-    launch_env_step32(h->dc, h->s32, a_dev, nullptr, nullptr, nullptr, nullptr, h->stream, m_out, h->d_bits, mode == 2);
+    launch_env_step32(h->dc, h->s32, a_dev, nullptr, nullptr, nullptr, nullptr, h->stream, m_out, h->d_bits, mode == 2,
+                      h->per_env());
     h->launches++;
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(done_bits, h->d_bits, sizeof(uint32_t) * nw, cudaMemcpyDeviceToHost, h->stream));
@@ -656,7 +662,8 @@ extern "C" int b747_step_host_packed(b747_handle* h, const float* act, float* ou
   rc = issue_pipeline(h, h->stream, in, outs, 2, chunks, per, [&](int lo, int hi, cudaStream_t s) {
     DevCfg dc = h->dc;
     dc.env_lo = lo; dc.env_hi = hi;
-    launch_env_step32(dc, h->s32, (const float*)h->d_act, nullptr, nullptr, nullptr, nullptr, s, h->d_out4, h->d_bits);
+    launch_env_step32(dc, h->s32, (const float*)h->d_act, nullptr, nullptr, nullptr, nullptr, s, h->d_out4, h->d_bits, false,
+                      h->per_env());
     h->launches++;
   });
   if (rc != B747_OK) return rc;
@@ -677,7 +684,7 @@ extern "C" int b747_model_step(b747_handle* h, int32_t n_steps) {
   if (!h || n_steps < 0) return fail(B747_ERR_ARG, "bad argument");
   CU(cudaSetDevice(h->cfg.device));
   if (h->cfg.dtype != B747_F64) return fail(B747_ERR_STATE, "raw model stepping needs an f64 handle (the reference's real_T is double)");
-  launch_model_step64(h->dc, h->s64, n_steps, h->stream);
+  launch_model_step64(h->dc, h->s64, n_steps, h->stream, h->per_env());
   h->launches++;
   CU(cudaGetLastError());
   return B747_OK;
@@ -690,6 +697,128 @@ extern "C" int b747_model_initialize(b747_handle* h) {
   launch_model_init64(h->dc, h->s64, h->stream);
   h->launches++;
   CU(cudaGetLastError());
+  return B747_OK;
+}
+
+// ---- per-env model tunables ---------------------------------------------------------------------
+// name -> first row (EnvParamRow) and component count; -1 for a name that is not per-env
+static const struct { const char* name; int row, n_comp; } kEnvParams[] = {
+    {"m0", EP_m0, 1}, {"Iz", EP_Iz, 1}, {"P", EP_P, 1}, {"S", EP_S, 1}, {"c_", EP_c, 1}, {"PID_SS", EP_PID_SS, 4},
+    {"PID_CS", EP_PID_CS, 4}};
+static int env_param_row(const char* name, int& n_comp) {
+  for (const auto& e : kEnvParams)
+    if (!strcmp(e.name, name)) { n_comp = e.n_comp; return e.row; }
+  n_comp = 0;
+  return -1;
+}
+
+// every env's rows [row, row + n_comp) <- v, and the float rows of f32 handles
+static int env_param_broadcast(b747_handle* h, int row, int n_comp, const double* v) {
+  const size_t np = (size_t)h->dc.n_pad;
+  double w[4] = {0, 0, 0, 0};
+  for (int j = 0; j < n_comp; j++) w[j] = v[j];
+  launch_env_param_fill(h->pe, h->cfg.n_envs, np, row, n_comp, w, h->stream);
+  h->launches++;
+  if (h->cfg.dtype == B747_F32) {
+    launch_env_param_derive32(h->pe, np, nullptr, h->cfg.n_envs, h->cfg.n_envs, h->stream);
+    h->launches++;
+  }
+  CU(cudaGetLastError());
+  return B747_OK;
+}
+
+static double* param_ptr(ModelParams& mp, const char* name, int& n);
+
+// per-env mode, entered for good: allocate the rows and give every env the batch values
+static int enter_per_env(b747_handle* h) {
+  if (h->pe.rows) return B747_OK;
+  const size_t np = (size_t)h->dc.n_pad;
+  EnvParams p;
+  bool ok = cudaMalloc(&p.rows, sizeof(double) * NEP * np) == cudaSuccess;
+  if (ok && h->cfg.dtype == B747_F32)
+    ok = cudaMalloc(&p.phys, sizeof(float4) * np) == cudaSuccess && cudaMalloc(&p.ss, sizeof(float4) * np) == cudaSuccess;
+  if (!ok) {
+    const std::string msg = cudaGetErrorString(cudaGetLastError());
+    cudaFree(p.rows); cudaFree(p.phys); cudaFree(p.ss);
+    return fail(B747_ERR_ALLOC, "per-env parameter rows: " + msg);
+  }
+  h->pe = p;
+  h->epoch++;  // the step kernels change
+  for (const auto& e : kEnvParams) {
+    int len;
+    const int rc = env_param_broadcast(h, e.row, e.n_comp, param_ptr(h->dc.mp, e.name, len));
+    if (rc != B747_OK) return rc;
+  }
+  return B747_OK;
+}
+
+// the index / value conventions of b747_save_state: int32 device indices (4-byte aligned), double values (8-byte aligned),
+// n <= n_envs without an index array
+static int env_param_args(b747_handle* h, const char* name, const double* vals, const int32_t* idx, int32_t n, int& row,
+                          int& n_comp) {
+  if (!h || !name || n < 0 || (n > 0 && !vals)) return fail(B747_ERR_ARG, "bad argument");
+  row = env_param_row(name, n_comp);
+  if (row < 0) return fail(B747_ERR_ARG, std::string("not a per-env parameter: ") + name);
+  if (!idx && n > h->cfg.n_envs) return fail(B747_ERR_ARG, "n > n_envs without an index array");
+  if ((uintptr_t)vals & 7) return fail(B747_ERR_ARG, "value arrays must be 8-byte aligned");
+  if ((uintptr_t)idx & 3) return fail(B747_ERR_ARG, "index arrays must be 4-byte aligned");
+  return B747_OK;
+}
+
+extern "C" int b747_set_env_param(b747_handle* h, const char* name, const double* values_dev, const int32_t* env_idx_dev,
+                                  int32_t n) {
+  int row, n_comp;
+  if (const int rc = env_param_args(h, name, values_dev, env_idx_dev, n, row, n_comp)) return rc;
+  CU(cudaSetDevice(h->cfg.device));
+  if (const int rc = enter_per_env(h)) return rc;
+  const size_t np = (size_t)h->dc.n_pad;
+  const double none[4] = {0, 0, 0, 0};
+  launch_env_param_io(h->pe, np, row, n_comp, env_idx_dev, n, h->cfg.n_envs, (double*)values_dev, true, none, h->stream);
+  h->launches++;
+  if (h->cfg.dtype == B747_F32 && n > 0) {
+    launch_env_param_derive32(h->pe, np, env_idx_dev, n, h->cfg.n_envs, h->stream);
+    h->launches++;
+  }
+  CU(cudaGetLastError());
+  return B747_OK;
+}
+
+extern "C" int b747_get_env_param(b747_handle* h, const char* name, const int32_t* env_idx_dev, int32_t n, double* out_dev) {
+  int row, n_comp;
+  if (const int rc = env_param_args(h, name, out_dev, env_idx_dev, n, row, n_comp)) return rc;
+  CU(cudaSetDevice(h->cfg.device));
+  int len;
+  const double* batch = param_ptr(h->dc.mp, name, len);
+  double b[4] = {0, 0, 0, 0};
+  for (int j = 0; j < n_comp; j++) b[j] = batch[j];
+  launch_env_param_io(h->pe, (size_t)h->dc.n_pad, row, n_comp, env_idx_dev, n, h->cfg.n_envs, out_dev, false, b, h->stream);
+  h->launches++;
+  CU(cudaGetLastError());
+  return B747_OK;
+}
+
+extern "C" int b747_set_env_param_range(b747_handle* h, const char* name, const double* lo, const double* hi, int n_comp) {
+  if (!h || !name) return fail(B747_ERR_ARG, "null argument");
+  int nc;
+  const int row = env_param_row(name, nc);
+  if (row < 0) return fail(B747_ERR_ARG, std::string("not a per-env parameter: ") + name);
+  if (n_comp != nc) return fail(B747_ERR_ARG, std::string("wrong number of components for ") + name);
+  if (!lo != !hi) return fail(B747_ERR_ARG, "lo and hi must both be given or both be NULL");
+  // mass, inertia, wing area and chord divide or scale every force: a draw must stay > 0
+  const bool positive = row == EP_m0 || row == EP_Iz || row == EP_S || row == EP_c;
+  for (int j = 0; lo && j < nc; j++) {
+    if (!isfinite(lo[j]) || !isfinite(hi[j])) return fail(B747_ERR_ARG, std::string("range bound is not finite: ") + name);
+    if (lo[j] > hi[j]) return fail(B747_ERR_ARG, std::string("range has lo > hi: ") + name);
+    if (positive && lo[j] <= 0.0) return fail(B747_ERR_ARG, std::string("range of ") + name + " must be > 0");
+  }
+  CU(cudaSetDevice(h->cfg.device));
+  if (const int rc = enter_per_env(h)) return rc;
+  for (int j = 0; j < nc; j++) {
+    const uint32_t bit = 1u << (row + j);
+    if (lo) { h->pe.lo[row + j] = lo[j]; h->pe.hi[row + j] = hi[j]; h->pe.ranged |= bit; }
+    else h->pe.ranged &= ~bit;
+  }
+  h->epoch++;  // launch arguments changed
   return B747_OK;
 }
 
@@ -716,6 +845,12 @@ extern "C" int b747_set_param(b747_handle* h, const char* name, const double* v,
   if (!p || n != len) return fail(B747_ERR_ARG, std::string("unknown parameter or wrong length: ") + name);
   memcpy(p, v, sizeof(double) * len);
   h->epoch++;  // launch arguments changed: captured pipelines are stale
+  int n_comp;
+  const int row = env_param_row(name, n_comp);
+  if (h->pe.rows && row >= 0) {  // per-env mode: the name's value of every env follows the batch value
+    CU(cudaSetDevice(h->cfg.device));
+    return env_param_broadcast(h, row, n_comp, v);
+  }
   return B747_OK;
 }
 extern "C" int b747_get_param(b747_handle* h, const char* name, double* v, int n) {

@@ -112,6 +112,28 @@ __host__ __device__ inline double uniform53(uint64_t seed, uint64_t env, uint32_
   return ((double)a * 67108864.0 + (double)b) * (1.0 / 9007199254740992.0);
 }
 
+// Per-env model tunables (b747_set_env_param): a handle in per-env mode owns field-major double rows [NEP][n_pad] in this
+// order, and f32 handles also the float rows the f32 twins read (mp32_phys, b747_model_mx.cuh).  A random reset of env i
+// draws row k, when it has a range, as lo + (hi - lo) * uniform53(seed, env_id_offset + i, episode, kEnvParamDraw0 + k),
+// with the episode index of the reset -- draw indices no episode draw uses (draw_episode stops at 19).
+enum EnvParamRow { EP_m0 = 0, EP_Iz, EP_P, EP_S, EP_c, EP_PID_SS, EP_PID_CS = EP_PID_SS + 4, NEP = EP_PID_CS + 4 };
+constexpr uint32_t kEnvParamDraw0 = 32;
+struct EnvParams {
+  double* rows = nullptr;  // [NEP][n_pad]
+  float4* phys = nullptr;  // f32 handles: [n_pad] (P / m0, P134 S / m0, P135 S c_ / Iz, 0)
+  float4* ss = nullptr;    // f32 handles: [n_pad] PID_SS rounded to float
+  double lo[NEP], hi[NEP];
+  uint32_t ranged = 0;     // bit k: row k is redrawn at every random reset
+};
+
+// the ranged rows of env i for episode epi (lo + (hi - lo) u rounded as written: no contraction into an FMA)
+__device__ inline void draw_env_params(const EnvParams& p, uint64_t seed, uint64_t env, uint32_t epi, size_t np, int i) {
+#pragma unroll
+  for (int k = 0; k < NEP; k++)
+    if ((p.ranged >> k) & 1u)
+      p.rows[(size_t)k * np + i] = __dadd_rn(p.lo[k], __dmul_rn(p.hi[k] - p.lo[k], uniform53(seed, env, epi, kEnvParamDraw0 + k)));
+}
+
 // Per-episode reference / initial condition in registers (Controller.reset's decisions).
 struct Episode {
   double s0[6];

@@ -85,11 +85,15 @@ bool f32_needs_cs(const DevCfg& c);
 void f32_warm_launch();
 // out4 != nullptr: packed outputs (one float4 = obs[3] + reward per env, done flags as one bit per env in done_bits);
 // obs / rew / done / term_obs are then unused.  prefetch_actions: `actions` is host-mapped memory.
+// pe: the handle's per-env tunables (b747_set_env_param), nullptr outside per-env mode.
 void launch_env_step32(const DevCfg& c, const StateF32& st, const float* actions, float* obs, float* rew, uint8_t* done,
                        float* term_obs, cudaStream_t s, float4* out4 = nullptr, uint32_t* done_bits = nullptr,
-                       bool prefetch_actions = false);
+                       bool prefetch_actions = false, const EnvParams* pe = nullptr);
+// random resets (eps == nullptr) of a handle with parameter ranges also draw the ranged rows of pe
 void launch_reset32(const DevCfg& c, const StateF32& st, const uint8_t* mask, const b747_episode* eps, float* obs,
-                    cudaStream_t s);
+                    cudaStream_t s, const EnvParams* pe = nullptr);
+// the float rows of envs env_idx[k] (nullptr: k) for k < n, recomputed from their double rows
+void launch_env_param_derive32(const EnvParams& pe, size_t np, const int32_t* env_idx, int n, int n_envs, cudaStream_t s);
 void launch_defaults32(const DevCfg& c, const StateF32& st, cudaStream_t s);
 // Storage kind of a per-env field of b747_get_field / b747_set_field (field table in b747_capi.cu).
 enum FieldKind { FK_SLOT, FK_STATE0, FK_SIG, FK_TICK, FK_FLAGS, FK_EPIDX, FK_LASTRET, FK_LASTLEN, FK_MXONLY };
@@ -97,10 +101,17 @@ int f32_field_io(const DevCfg& c, StateF32& s, FieldKind kind, int row, const ch
                  cudaStream_t stream);
 
 void launch_env_step64(const DevCfg& c, const StateF64& st, const double* actions, double* obs, double* rew,
-                       uint8_t* done, double* term_obs, cudaStream_t s);
-void launch_model_step64(const DevCfg& c, const StateF64& st, int n_steps, cudaStream_t s);
+                       uint8_t* done, double* term_obs, cudaStream_t s, const EnvParams* pe = nullptr);
+void launch_model_step64(const DevCfg& c, const StateF64& st, int n_steps, cudaStream_t s, const EnvParams* pe = nullptr);
 void launch_reset64(const DevCfg& c, const StateF64& st, const uint8_t* mask, const b747_episode* eps, double* obs,
-                    cudaStream_t s);
+                    cudaStream_t s, const EnvParams* pe = nullptr);
+// b747_set_env_param / b747_get_env_param: rows [row0, row0 + n_comp) of envs env_idx[k] (nullptr: k) <-> vals[k][n_comp]
+// (out-of-range entries skip k).  Outside per-env mode (pe.rows == nullptr) a get returns `batch`.
+void launch_env_param_io(const EnvParams& pe, size_t np, int row0, int n_comp, const int32_t* env_idx, int n, int n_envs,
+                         double* vals, bool set, const double batch[4], cudaStream_t s);
+// every env's rows [row0, row0 + n_comp) <- v (entering per-env mode, b747_set_param in per-env mode)
+void launch_env_param_fill(const EnvParams& pe, int n_envs, size_t np, int row0, int n_comp, const double v[4],
+                           cudaStream_t s);
 void launch_defaults64(const DevCfg& c, const StateF64& st, cudaStream_t s);
 void launch_model_init64(const DevCfg& c, const StateF64& st, cudaStream_t s);
 // calc_stepinfo's final arithmetic on the tracker (snapshot != 0: the last finished episode): out[env][5] =

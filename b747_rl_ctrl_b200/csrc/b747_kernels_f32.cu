@@ -217,6 +217,33 @@ __device__ __forceinline__ void load_tables32(float4* sT, const float4* __restri
   __syncthreads();
 }
 
+// per-env twins: the env's tunables into registers (32 B; + 32 B of PID_CS with the altitude loop)
+template <bool CS>
+__device__ __forceinline__ void load_env_params_mx(const EnvParams& pe, size_t np, int i, RegsMx& r) {
+  const float4 ph = pe.phys[i], ss = pe.ss[i];
+  r.pe.P_m = ph.x; r.pe.kS_m = ph.y; r.pe.half_Sc_over_Iz = ph.z;
+  r.pe.PID_SS[0] = ss.x; r.pe.PID_SS[1] = ss.y; r.pe.PID_SS[2] = ss.z; r.pe.PID_SS[3] = ss.w;
+  if (CS) {
+#pragma unroll
+    for (int k = 0; k < 4; k++) r.pe_cs[k] = pe.rows[(size_t)(EP_PID_CS + k) * np + i];
+  }
+}
+
+// the float rows of env i from its double rows (mp32_phys: the host's MP32 derivation)
+__device__ __forceinline__ void derive_env_params_mx(const EnvParams& pe, size_t np, int i) {
+  const double* R = pe.rows;
+#define EPV(k) R[(size_t)(k) * np + i]
+  pe.phys[i] = mp32_phys(EPV(EP_P), EPV(EP_m0), EPV(EP_S), EPV(EP_c), EPV(EP_Iz));
+  pe.ss[i] = make_float4((float)EPV(EP_PID_SS), (float)EPV(EP_PID_SS + 1), (float)EPV(EP_PID_SS + 2), (float)EPV(EP_PID_SS + 3));
+#undef EPV
+}
+
+// a random reset of env i (episode index epi): new ranged rows and the float rows that follow from them
+__device__ __noinline__ void redraw_env_params_mx(const EnvParams& pe, const DevCfg& c, size_t np, int i, uint32_t epi) {
+  draw_env_params(pe, c.seed, (uint64_t)(c.env_id_offset + i), epi, np, i);
+  derive_env_params_mx(pe, np, i);
+}
+
 // ------------------------------------------------------------------------------------------
 constexpr int kStepThreads = 128, kStepWarps = kStepThreads / 32;  // threads per block of every step kernel tier
 constexpr int kF32MinBlocks = 4;  // measured: 4 x 128 threads at 126 registers, no spills, beats every other occupancy point
@@ -224,17 +251,26 @@ constexpr int kExtMinBlocks = 3;
 constexpr int kGenMinBlocks = 3;  // measured: 168 registers x 12 warps beats 242 x 8 (0.66 -> 0.52 ms per 1 Mi-env K=10 step)
 // TIER 0: canonical family (LEAN layout); 1: general layout without the altitude loop (other observation layouts,
 // oscillating references, aero disturbance, TF reward); 2: + the altitude loop (СУ PID); 3: + recorder, tracker, signal export.
+// TIER | kTierPE (5, 6, 7): the per-env twin of tier 1, 2, 3 -- the same pass reading PID_SS, P / m0, P134 S / m0,
+// P135 S c_ / Iz (and PID_CS with the altitude loop) from the env's rows in `pe`, loaded with the tile's state, instead of
+// from the launch; done envs redraw their ranged rows.  The flag rides in TIER so that the other instantiations keep
+// their names.
 // PFA: the next tile's actions are fetched while the current tile is stepped (host-mapped action buffers: a PCIe read
 // has ~2 us of latency, a tile at K = 10 takes ~20 us).
+constexpr int kTierPE = 4;
 template <int TIER, int SW = -1, bool STG = false, bool PFA = false>
-__global__ void __launch_bounds__(kStepThreads, TIER >= 2 ? kGenMinBlocks : (TIER == 1 ? kExtMinBlocks : kF32MinBlocks))
+__global__ void __launch_bounds__(kStepThreads, (TIER & 3) >= 2 ? kGenMinBlocks : ((TIER & 3) == 1 ? kExtMinBlocks : kF32MinBlocks))
 k_env_step32(DevCfg c, MP32 mp, StateF32 st, const float* __restrict__ actions, float* __restrict__ obs_out,
              float* __restrict__ rew_out, uint8_t* __restrict__ done_out, float* __restrict__ term_obs,
-             float4* __restrict__ out4, uint32_t* __restrict__ done_bits, unsigned int* __restrict__ tile_ctr) {
+             float4* __restrict__ out4, uint32_t* __restrict__ done_bits, unsigned int* __restrict__ tile_ctr,
+             const __grid_constant__ EnvParams pe) {
   // Persistent warps: the launch fills the GPU once (blocks = SMs x resident blocks per SM), the tables are staged into
   // shared memory once per block, and every warp then walks its own stride of 32-env tiles with no block-level
   // synchronisation until the episode statistics are flushed at the very end.
-  constexpr bool GEN = TIER >= 1, CS = TIER >= 2, TRACE = TIER >= 3;
+  constexpr int T = TIER & 3;
+  constexpr bool PE = (TIER & kTierPE) != 0;
+  static_assert(!PE || (T >= 1 && SW < 0 && !STG && !PFA), "per-env twins exist for the general tiers only");
+  constexpr bool GEN = T >= 1, CS = T >= 2, TRACE = T >= 3;
   constexpr bool STAGED = !GEN && STG;
   __shared__ float4 sT[kFastCells];
   __shared__ double s_stats[4];
@@ -295,6 +331,7 @@ k_env_step32(DevCfg c, MP32 mp, StateF32 st, const float* __restrict__ actions, 
       load_mx<GEN, CS>(st.D, st.F, np, i, r);
       if (!PFA) a = actions[i];
     }
+    if (PE) load_env_params_mx<CS>(pe, np, i, r);
     if (c.norm_act) a *= (float)c.action_max;
     const bool use_ctrl = CS && (r.flags & FL_USE_CTRL);
     // Controller.step: reference, then the action law (core/controller.py:233-251)
@@ -324,7 +361,7 @@ k_env_step32(DevCfg c, MP32 mp, StateF32 st, const float* __restrict__ actions, 
     const bool want_x = GEN && (c.obs_type == B747_OBS_MODEL_STATE || tracing);
 #pragma unroll 1
     for (int k = 0; k < c.substeps; k++) {
-      model_step32<TIER, SW>(sT, mp, c, r, o, s4, want_x);
+      model_step32<T, SW, PE>(sT, mp, c, r, o, s4, want_x);
       if (TRACE && tracing) {  // Controller._post_step (core/controller.py:209-228)
         TraceSample ts;
         ts.t = (double)r.tick * kH; ts.U_com = o.U_com; ts.U_PID = o.U_com_PID; ts.deltaz_RP = o.deltaz_RP;
@@ -464,7 +501,11 @@ k_env_step32(DevCfg c, MP32 mp, StateF32 st, const float* __restrict__ actions, 
         if (TRACE) trace_clear(st.trace, np, i);
         Episode ep;
         if (c.reset_ref_mode == B747_RESET_NONE) episode_from_state_mx(st, np, i, r, ep);
-        else { draw_episode(c, (uint64_t)(c.env_id_offset + i), r.ep_idx, ep); r.ep_idx++; }
+        else {
+          draw_episode(c, (uint64_t)(c.env_id_offset + i), r.ep_idx, ep);
+          if (PE && pe.ranged) redraw_env_params_mx(pe, c, np, i, r.ep_idx);
+          r.ep_idx++;
+        }
         env_reset_mx<GEN>(c, ep, r, st, np, i);
         full_store = true;
         for (int k = 0; k < od; k++) obs[k] = 0.f;
@@ -518,6 +559,27 @@ __global__ void __launch_bounds__(128) k_reset32(DevCfg c, StateF32 st, const ui
   store_mx<GEN>(st, np, i, r, true);
 }
 
+// b747_reset of a handle with parameter ranges: the ranged rows of the envs about to draw a new episode, with the episode
+// index k_reset32 is about to use (launched just before it)
+__global__ void __launch_bounds__(128) k_env_param_draw32(DevCfg c, StateF32 st, const __grid_constant__ EnvParams pe,
+                                                          const uint8_t* __restrict__ mask) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= c.n_envs || (mask && !mask[i])) return;
+  const size_t np = (size_t)c.n_pad;
+  const uint32_t epi = __float_as_uint(st.F[FG_misc * np + i].w) >> 8;
+  redraw_env_params_mx(pe, c, np, i, epi);
+}
+
+// b747_set_env_param / b747_set_param of an f32 handle in per-env mode: the float rows of the written envs
+__global__ void __launch_bounds__(128) k_env_param_derive32(EnvParams pe, size_t np, const int32_t* __restrict__ env_idx,
+                                                            int n, int n_envs) {
+  const int k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  const int i = env_idx ? env_idx[k] : k;
+  if (i < 0 || i >= n_envs) return;
+  derive_env_params_mx(pe, np, i);
+}
+
 __global__ void __launch_bounds__(128) k_defaults32(DevCfg c, StateF32 st) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= c.n_pad) return;
@@ -553,9 +615,10 @@ bool f32_needs_cs(const DevCfg& c) {
 static MP32 make_mp32(const ModelParams& m) {
   MP32 p;
   for (int k = 0; k < 4; k++) p.PID_SS[k] = (float)m.PID_SS[k];
-  p.P_m = (float)(m.P / m.m0); p.g = (float)m.g;
-  p.kS_m = (float)(Pc(134) * m.S / m.m0);
-  p.half_Sc_over_Iz = (float)(Pc(135) * m.S * m.c_ / m.Iz);
+  const float4 ph = mp32_phys(m.P, m.m0, m.S, m.c_, m.Iz);
+  p.P_m = ph.x; p.g = (float)m.g;
+  p.kS_m = ph.y;
+  p.half_Sc_over_Iz = ph.z;
   p.sw = (m.use_RL >= Pc(148) ? SW_RL : 0) | (m.use_PID_SS >= Pc(9) ? SW_SS : 0) | (m.use_RP >= Pc(149) ? SW_RP : 0) |
          (m.use_PID_SS != 0.0 ? SW_SS_ON : 0);
   return p;
@@ -623,15 +686,17 @@ void f32_warm_launch() {
   const int big = 1 << 30;
   step_grid<0, SW_RP, false, true>(big); step_grid<0, SW_RP, true>(big); step_grid<0, SW_RP>(big); step_grid<0>(big);
   step_grid<1, SW_RP>(big); step_grid<1>(big); step_grid<2>(big); step_grid<3>(big);
+  step_grid<1 | kTierPE>(big); step_grid<2 | kTierPE>(big); step_grid<3 | kTierPE>(big);
 }
 
 void launch_env_step32(const DevCfg& c, const StateF32& st, const float* actions, float* obs, float* rew, uint8_t* done,
-                       float* term_obs, cudaStream_t s, float4* out4, uint32_t* done_bits, bool prefetch_actions) {
+                       float* term_obs, cudaStream_t s, float4* out4, uint32_t* done_bits, bool prefetch_actions,
+                       const EnvParams* pe) {
   const MP32 mp = make_mp32(c.mp);
   const int n = c.env_hi - c.env_lo;
   if (n <= 0) return;
   const bool plain = !st.trace.trk && !st.trace.rec && !st.sig && !c.force_full;
-  const bool lean = plain && f32_is_lean(c);
+  const bool lean = plain && f32_is_lean(c) && !pe;  // per-env mode: a canonical configuration runs the tier-1 twin
   const bool lean_rp = lean && mp.sw == SW_RP;  // the canonical switch setting (use_RP only) as a compile-time constant
   const bool staged = lean_rp && !prefetch_actions && c.substeps <= kStagedMaxK;  // HBM-bound regime: TMA-staged state
   // tile counter of this launch: one of kTileCtrSlots words, zeroed on the launch stream (launches of one handle may
@@ -644,8 +709,14 @@ void launch_env_step32(const DevCfg& c, const StateF32& st, const float* actions
   }
 #define B747_LAUNCH(TIER, ...) \
   k_env_step32<TIER, ##__VA_ARGS__><<<step_grid<TIER, ##__VA_ARGS__>(n), kStepThreads, 0, s>>>( \
-      c, mp, st, actions, obs, rew, done, term_obs, out4, done_bits, ctr)
-  if (lean_rp && prefetch_actions)  // host-mapped action buffer (b747_step_host_packed)
+      c, mp, st, actions, obs, rew, done, term_obs, out4, done_bits, ctr, pe ? *pe : EnvParams{})
+  if (pe && plain && !f32_needs_cs(c))
+    B747_LAUNCH(1 | kTierPE);
+  else if (pe && plain)
+    B747_LAUNCH(2 | kTierPE);
+  else if (pe)
+    B747_LAUNCH(3 | kTierPE);
+  else if (lean_rp && prefetch_actions)  // host-mapped action buffer (b747_step_host_packed)
     B747_LAUNCH(0, SW_RP, false, true);
   else if (staged)
     B747_LAUNCH(0, SW_RP, true);
@@ -664,9 +735,14 @@ void launch_env_step32(const DevCfg& c, const StateF32& st, const float* actions
 #undef B747_LAUNCH
 }
 void launch_reset32(const DevCfg& c, const StateF32& st, const uint8_t* mask, const b747_episode* eps, float* obs,
-                    cudaStream_t s) {
+                    cudaStream_t s, const EnvParams* pe) {
+  if (pe && pe->ranged && !eps && c.reset_ref_mode != B747_RESET_NONE)
+    k_env_param_draw32<<<grid_for(c.n_envs, 128), 128, 0, s>>>(c, st, *pe, mask);
   // resets always go through the general layout so that every group is initialised
   k_reset32<true><<<grid_for(c.n_envs, 128), 128, 0, s>>>(c, st, mask, eps, obs);
+}
+void launch_env_param_derive32(const EnvParams& pe, size_t np, const int32_t* env_idx, int n, int n_envs, cudaStream_t s) {
+  if (n > 0) k_env_param_derive32<<<grid_for(n, 128), 128, 0, s>>>(pe, np, env_idx, n, n_envs);
 }
 void launch_defaults32(const DevCfg& c, const StateF32& st, cudaStream_t s) {
   k_defaults32<<<grid_for(c.n_pad, 128), 128, 0, s>>>(c, st);

@@ -177,13 +177,27 @@ __device__ __forceinline__ void load_tables64(double* sP) {
   __syncthreads();
 }
 
+// per-env twins (PE): the launch's tunables with this env's rows in place of the per-env names
+__device__ __forceinline__ void env_params64(const EnvParams& pe, const ModelParams& batch, size_t np, int i, ModelParams& mp) {
+  mp = batch;
+  const double* R = pe.rows;
+#define EPV(k) R[(size_t)(k) * np + i]
+  mp.m0 = EPV(EP_m0); mp.Iz = EPV(EP_Iz); mp.P = EPV(EP_P); mp.S = EPV(EP_S); mp.c_ = EPV(EP_c);
+#pragma unroll
+  for (int k = 0; k < 4; k++) { mp.PID_SS[k] = EPV(EP_PID_SS + k); mp.PID_CS[k] = EPV(EP_PID_CS + k); }
+#undef EPV
+}
+
 // ------------------------------------------------------------------------------------------
-// ControllerEnv.step for every env of the handle.
+// ControllerEnv.step for every env of the handle.  PE: the per-env twin, which reads the tunables from the env's rows
+// in `pe` and redraws the ranged ones at an auto-reset.
 // ------------------------------------------------------------------------------------------
 constexpr int kF64MinBlocks = 2;  // measured: beats 3 / 4 blocks at 168 / 128 registers (1.783 vs 2.04-2.22 ms: spills)
+template <bool PE>
 __global__ void __launch_bounds__(128, kF64MinBlocks) k_env_step64(DevCfg c, StateF64 st, const double* __restrict__ actions,
                                                     double* __restrict__ obs_out, double* __restrict__ rew_out,
-                                                    uint8_t* __restrict__ done_out, double* __restrict__ term_obs) {
+                                                    uint8_t* __restrict__ done_out, double* __restrict__ term_obs,
+                                                    const __grid_constant__ EnvParams pe) {
   __shared__ double sP[kNP];
   __shared__ EpStatsSmem sst;
   load_tables64(sP);
@@ -195,6 +209,9 @@ __global__ void __launch_bounds__(128, kF64MinBlocks) k_env_step64(DevCfg c, Sta
   if (live) {
     Regs64 r;
     load_regs64(st.slots, st.tick, st.flags, st.ep_idx, np, i, r);
+    ModelParams mpe;
+    if (PE) env_params64(pe, c.mp, np, i, mpe);
+    const ModelParams& mp = PE ? mpe : c.mp;
     Pass64 o;
     double Xs4[16];
     double a = actions[i];
@@ -224,7 +241,7 @@ __global__ void __launch_bounds__(128, kF64MinBlocks) k_env_step64(DevCfg c, Sta
     const bool tracing = st.trace.trk || st.trace.rec;
 #pragma unroll 1
     for (int k = 0; k < c.substeps; k++) {
-      model_step64(sP, c.mp, r, o, Xs4);
+      model_step64(sP, mp, r, o, Xs4);
       if (tracing) {  // Controller._post_step (core/controller.py:209-228)
         TraceSample ts;
         ts.t = (double)r.tick * kH; ts.U_com = o.U_com; ts.U_PID = o.U_com_PID; ts.deltaz_RP = o.deltaz_RP;
@@ -261,7 +278,11 @@ __global__ void __launch_bounds__(128, kF64MinBlocks) k_env_step64(DevCfg c, Sta
         trace_clear(st.trace, np, i);
         Episode ep;
         if (c.reset_ref_mode == B747_RESET_NONE) episode_from_slots(st.slots, np, i, r, ep);
-        else { draw_episode(c, (uint64_t)(c.env_id_offset + i), r.ep_idx, ep); r.ep_idx++; }
+        else {
+          draw_episode(c, (uint64_t)(c.env_id_offset + i), r.ep_idx, ep);
+          if (PE) draw_env_params(pe, c.seed, (uint64_t)(c.env_id_offset + i), r.ep_idx, np, i);
+          r.ep_idx++;
+        }
         env_reset64(c, sP, ep, r, st.slots, np, i);
         for (int k = 0; k < od; k++) obs[k] = 0.0;  // every exported signal is zero after initialize
         if (st.sig) for (int k = 0; k < NSIG; k++) st.sig[(size_t)k * np + i] = 0.0;
@@ -273,8 +294,9 @@ __global__ void __launch_bounds__(128, kF64MinBlocks) k_env_step64(DevCfg c, Sta
   block_episode_stats(sst, done, ep_ret, ep_len, st.stats);
 }
 
-// Model.step x n_steps (core/model.py:247-250): no action law, no reward.
-__global__ void __launch_bounds__(128) k_model_step64(DevCfg c, StateF64 st, int n_steps) {
+// Model.step x n_steps (core/model.py:247-250): no action law, no reward.  PE: per-env twin.
+template <bool PE>
+__global__ void __launch_bounds__(128) k_model_step64(DevCfg c, StateF64 st, int n_steps, const __grid_constant__ EnvParams pe) {
   __shared__ double sP[kNP];
   load_tables64(sP);
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -282,13 +304,25 @@ __global__ void __launch_bounds__(128) k_model_step64(DevCfg c, StateF64 st, int
   const size_t np = (size_t)c.n_pad;
   Regs64 r;
   load_regs64(st.slots, st.tick, st.flags, st.ep_idx, np, i, r);
+  ModelParams mpe;
+  if (PE) env_params64(pe, c.mp, np, i, mpe);
+  const ModelParams& mp = PE ? mpe : c.mp;
   Pass64 o;
   double Xs4[16];
 #pragma unroll 1
-  for (int k = 0; k < n_steps; k++) model_step64(sP, c.mp, r, o, Xs4);
+  for (int k = 0; k < n_steps; k++) model_step64(sP, mp, r, o, Xs4);
   r.sig_upid = o.U_com_PID; r.sig_vzh = o.vartheta_zh;
   if (st.sig) export_signals64(st.sig, np, i, r, o, Xs4, (double)r.tick * kH);
   store_regs64(st.slots, st.tick, st.flags, st.ep_idx, np, i, r);
+}
+
+// b747_reset of a handle with parameter ranges: the ranged rows of the envs about to draw a new episode, with the episode
+// index k_reset64 is about to use (launched just before it)
+__global__ void __launch_bounds__(128) k_env_param_draw64(DevCfg c, StateF64 st, const __grid_constant__ EnvParams pe,
+                                                          const uint8_t* __restrict__ mask) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= c.n_envs || (mask && !mask[i])) return;
+  draw_env_params(pe, c.seed, (uint64_t)(c.env_id_offset + i), st.ep_idx[i], (size_t)c.n_pad, i);
 }
 
 // Controller.reset + ControllerEnv.reset: random draws (eps==nullptr) or explicit episodes.
@@ -388,16 +422,20 @@ void launch_transfer_metrics(const DevCfg& c, const TraceState& tr, int which, i
 }
 
 void launch_env_step64(const DevCfg& c, const StateF64& st, const double* actions, double* obs, double* rew,
-                       uint8_t* done, double* term_obs, cudaStream_t s) {
+                       uint8_t* done, double* term_obs, cudaStream_t s, const EnvParams* pe) {
   const int n = c.env_hi - c.env_lo;
   if (n <= 0) return;
-  k_env_step64<<<grid_for(n, 128), 128, 0, s>>>(c, st, actions, obs, rew, done, term_obs);
+  if (pe) k_env_step64<true><<<grid_for(n, 128), 128, 0, s>>>(c, st, actions, obs, rew, done, term_obs, *pe);
+  else k_env_step64<false><<<grid_for(n, 128), 128, 0, s>>>(c, st, actions, obs, rew, done, term_obs, EnvParams{});
 }
-void launch_model_step64(const DevCfg& c, const StateF64& st, int n_steps, cudaStream_t s) {
-  k_model_step64<<<grid_for(c.n_envs, 128), 128, 0, s>>>(c, st, n_steps);
+void launch_model_step64(const DevCfg& c, const StateF64& st, int n_steps, cudaStream_t s, const EnvParams* pe) {
+  if (pe) k_model_step64<true><<<grid_for(c.n_envs, 128), 128, 0, s>>>(c, st, n_steps, *pe);
+  else k_model_step64<false><<<grid_for(c.n_envs, 128), 128, 0, s>>>(c, st, n_steps, EnvParams{});
 }
 void launch_reset64(const DevCfg& c, const StateF64& st, const uint8_t* mask, const b747_episode* eps, double* obs,
-                    cudaStream_t s) {
+                    cudaStream_t s, const EnvParams* pe) {
+  if (pe && pe->ranged && !eps && c.reset_ref_mode != B747_RESET_NONE)
+    k_env_param_draw64<<<grid_for(c.n_envs, 128), 128, 0, s>>>(c, st, *pe, mask);
   k_reset64<<<grid_for(c.n_envs, 128), 128, 0, s>>>(c, st, mask, eps, obs);
 }
 void launch_defaults64(const DevCfg& c, const StateF64& st, cudaStream_t s) {

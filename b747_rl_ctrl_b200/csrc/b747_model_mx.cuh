@@ -83,6 +83,11 @@ struct MP32 {
   float P_m, g, kS_m, half_Sc_over_Iz;  // thrust / m0, g, P134 S / m0, P135 S c / Iz
   int sw;
 };
+// The three pre-divided floats of MP32 from the double tunables: double operations in this order, then rounded to float.
+// The host (whole-batch MP32) and the device (per-env rows) both use it, so equal values give equal floats.
+__host__ __device__ inline float4 mp32_phys(double P, double m0, double S, double c_, double Iz) {
+  return make_float4((float)(P / m0), (float)(Pc(134) * S / m0), (float)(Pc(135) * S * c_ / Iz), 0.f);
+}
 
 struct RegsMx {
   double h, th, Vx, Vy, wz, ssi, ssf, dvi, itse;  // integrator states, accumulated in float64
@@ -96,6 +101,8 @@ struct RegsMx {
   int tick, flags;
   uint32_t ep_idx;
   TabCache tc;                                     // look-up state (registers only; invalid at load: widths 0)
+  MP32 pe;                                         // per-env twins: this env's PID_SS, P_m, kS_m, half_Sc_over_Iz
+  double pe_cs[4];                                 // per-env twins with the altitude loop: this env's PID_CS
 };
 
 struct PassMx {
@@ -279,7 +286,8 @@ struct TrigMx { float2 sc, cn; float thf, sgn, ub, wb, rV, alpha; double thd; };
 // the pitch angle and the pitch error in float64 (th_d); the half-step passes only feed float32 RK4 sums and use th_f.
 // TIER 0: canonical (LEAN) model; 1: + aero-disturbance gains (general layout, no altitude loop); 2: + the altitude loop (СУ PID)
 // SW >= 0: the diagram's manual switches as a compile-time constant (the canonical env: SW_RP only); -1: read mp.sw
-template <int TIER, int SW = -1>
+// PE: per-env twin -- PID_SS, PID_CS, P_m, kS_m and half_Sc_over_Iz come from the env's registers (r.pe, r.pe_cs)
+template <int TIER, int SW = -1, bool PE = false>
 __device__ __forceinline__ void pass32(const float4* __restrict__ sT, const MP32& mp, const DevCfg& c, int stage, int n,
                                        double th_d, float dth, TrigMx& tg, float vref_f, float t_f, float h, double h_d, float Vx,
                                        float Vy, float wz, float ssi, float ssf, double csi, double csf, RegsMx& r,
@@ -287,6 +295,8 @@ __device__ __forceinline__ void pass32(const float4* __restrict__ sT, const MP32
                                        float& f_Vy, float& f_wz, float& f_ssi, float& f_ssf, double& f_csi, double& f_csf,
                                        float& f_itse) {
   constexpr bool GEN = TIER >= 1, CS = TIER >= 2;
+  const MP32& tun = PE ? r.pe : mp;  // the per-env tunables; g and the switches stay whole-batch (mp)
+  auto pid_cs = [&](int k) { return PE ? r.pe_cs[k] : c.mp.PID_CS[k]; };
   const bool major = stage == 0;
   const bool dbl = stage == 0 || stage == 3;
   // attitude.  Beyond +-90 deg the DLL's pitch asin(sin(theta)) folds back: with k = round(theta/pi) and
@@ -413,8 +423,8 @@ __device__ __forceinline__ void pass32(const float4* __restrict__ sT, const MP32
   // drag/lift rotated by alpha with sin(alpha) = -wb/V, cos(alpha) = ub/V gives
   //   Fx = q S (c_x ub - CYa wb)/V + P,  Fy = q S (CYa ub + c_x wb)/V,  q S / V = rho V S / 2,  c_x = P126 CXa
   const float rV2 = rho * V2;
-  const float kq = rV2 * (rV * mp.kS_m);
-  const float Fx = fmaf(kq, fmaf(-CYa, wb, cx * ub), mp.P_m);
+  const float kq = rV2 * (rV * tun.kS_m);
+  const float Fx = fmaf(kq, fmaf(-CYa, wb, cx * ub), tun.P_m);
   const float Fy = kq * fmaf(cx, wb, CYa * ub);
   // actuator: transport delay (3 steps) -> discrete filter (every 5th tick) -> rate limiter -> saturation
   float td;
@@ -440,8 +450,8 @@ __device__ __forceinline__ void pass32(const float4* __restrict__ sT, const MP32
   if (CS) {
     use_cs = (r.flags & FL_USE_CTRL) && (1.f >= PCF(146));
     e_h = r.href - h_d;  // h_zh - h
-    cs_d = (e_h * c.mp.PID_CS[2] - csf) * c.mp.PID_CS[3];
-    cs_pre = e_h * c.mp.PID_CS[0] + csi + cs_d;
+    cs_d = (e_h * pid_cs(2) - csf) * pid_cs(3);
+    cs_pre = e_h * pid_cs(0) + csi + cs_d;
     vzh_d = fmin(fmax(cs_pre, Pc(4)), Pc(6));
     o.vartheta_zh = __double2float_rn(vzh_d);
   } else {
@@ -458,8 +468,8 @@ __device__ __forceinline__ void pass32(const float4* __restrict__ sT, const MP32
   }
   o.dvf = dv;
   // СС PID
-  const float ss_d = (dv * mp.PID_SS[2] - ssf) * mp.PID_SS[3];
-  const float ss_pre = fmaf(dv, mp.PID_SS[0], ssi) + ss_d;
+  const float ss_d = (dv * tun.PID_SS[2] - ssf) * tun.PID_SS[3];
+  const float ss_pre = fmaf(dv, tun.PID_SS[0], ssi) + ss_d;
   o.U_com_PID = satf(ss_pre, PCF(5), PCF(7));
   const int sw = SW >= 0 ? SW : mp.sw;
   if (sw & SW_RL) o.U_com = PCF(147) > fabsf(o.U_com_PID) ? 0.f : o.U_com_PID;
@@ -468,10 +478,10 @@ __device__ __forceinline__ void pass32(const float4* __restrict__ sT, const MP32
   const float ay = fmaf(Fy, cs, fmaf(Fx, sn, -mp.g));
   const float dze = (sw & SW_RP) ? o.deltaz_RP : o.U_com;
   const float Cm = fmaf(dcm * Ka, dze, mz);
-  const float wzd = Cm * (rV2 * mp.half_Sc_over_Iz);
+  const float wzd = Cm * (rV2 * tun.half_Sc_over_Iz);
   // clamping anti-windup (СС)
   const float dz = ss_pre - o.U_com_PID;
-  float ss_i = mp.PID_SS[1] * dv;
+  float ss_i = tun.PID_SS[1] * dv;
   if (PCF(291) == 0.f)  // ZeroGain: ss_pre*0 != dz  <=>  dz != 0 (finite ss_pre); sign(dz)==sign(ss_i) via the sign bits
     o.and_ss = (dz != 0.f) & (ss_i != 0.f) & ((__float_as_int(dz) ^ __float_as_int(ss_i)) >= 0);
   else
@@ -482,7 +492,7 @@ __device__ __forceinline__ void pass32(const float4* __restrict__ sT, const MP32
   f_itse = dv * dv * t_f;
   if (CS) {
     const double dzc = cs_pre - vzh_d;
-    double cs_i = e_h * c.mp.PID_CS[1];
+    double cs_i = e_h * pid_cs(1);
     o.and_cs = (cs_pre * Pc(292) != dzc) && (((dzc > 0.0) - (dzc < 0.0)) == ((cs_i > 0.0) - (cs_i < 0.0)));
     if (major) memout_cs = (r.flags & FL_MEM_CS) != 0;
     if (memout_cs) cs_i = Pc(11);
@@ -494,7 +504,7 @@ __device__ __forceinline__ void pass32(const float4* __restrict__ sT, const MP32
 
 // model_simple_step in the mixed formulation.  On return r holds the post-update state, `o` the
 // stage-4 pass and s4 the stage-4 (predictor) state values.
-template <int TIER, int SW = -1>
+template <int TIER, int SW = -1, bool PE = false>
 __device__ __forceinline__ void model_step32(const float4* __restrict__ sT, const MP32& mp, const DevCfg& c, RegsMx& r,
                                              PassMx& o, Stage4Mx& s4, bool want_x) {
   constexpr bool CS = TIER >= 2;
@@ -525,7 +535,7 @@ __device__ __forceinline__ void model_step32(const float4* __restrict__ sT, cons
     const float t_f = s == 0 ? t0f : (s == 3 ? t0f + hh : t0f + hhalf);
     float f_h, f_Vx, f_Vy, f_wz, f_ssi, f_ssf, f_itse;
     double f_csi, f_csf;
-    pass32<TIER, SW>(sT, mp, c, s, n, X_th, d_th, tg, vref_f, t_f, X_h, Xd_h, XXI.x, XVW.x, XVW.y, XXI.y, X_ssf, X_csi, X_csf, r, at,
+    pass32<TIER, SW, PE>(sT, mp, c, s, n, X_th, d_th, tg, vref_f, t_f, X_h, Xd_h, XXI.x, XVW.x, XVW.y, XXI.y, X_ssf, X_csi, X_csf, r, at,
                 memout_ss, memout_cs, o, f_h, f_Vx, f_Vy, f_wz, f_ssi, f_ssf, f_csi, f_csf, f_itse);
     if (s == 0) {
       // update(): discrete filter, rate-limiter memory, Memory blocks, Derivative history, delay push

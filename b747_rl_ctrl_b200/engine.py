@@ -20,6 +20,9 @@ DIST_NONE, DIST_AERO = -1, 0
 OBS_PID_LIKE, OBS_SPEED_MODE, OBS_PID_AERO, OBS_PID_SPEED_AERO, OBS_MODEL_STATE = 0, 1, 2, 3, 4
 REW_CLASSIC, REW_PID_LIKE, REW_QUALITY, REW_MINIMAL, REW_TF_REFERENCE = 0, 1, 2, 3, 4
 OBS_DIM = {0: 3, 1: 5, 2: 8, 3: 10, 4: 7}
+# per-env model tunables (b747_set_env_param) and their component counts, in the order of their Philox draw indices
+ENV_PARAMS = {"m0": 1, "Iz": 1, "P": 1, "S": 1, "c_": 1, "PID_SS": 4, "PID_CS": 4}
+ENV_PARAM_DRAW0 = 32
 
 
 def make_cfg(n_envs, dtype=F32, device=0, obs_type=OBS_PID_LIKE, rew_type=REW_CLASSIC, ctrl_type=CTRL_MANUAL,
@@ -335,6 +338,54 @@ class BatchEngine:
         n = idx.numel() if idx is not None else (bidx.numel() if bidx is not None else self.n_envs)
         self._order(after_torch=True)
         check(self._L.b747_load_state(self._h, _ptr(b), _ptr(bidx), _ptr(idx), n))
+
+    # -- per-env model tunables (domain randomisation, gain sweeps) -------------------------------------------
+    def _env_param_n(self, name):
+        if name not in ENV_PARAMS:
+            raise KeyError(f"not a per-env parameter: {name} (one of {', '.join(ENV_PARAMS)})")
+        return ENV_PARAMS[name]
+
+    def set_env_param(self, name, values, indices=None):
+        """Env indices[k] (default: env k) takes values[k] ([n] or [n, 4] for PID_SS / PID_CS; numpy or a device
+        tensor).  The first call puts the handle in per-env mode for good, every env starting from the whole-batch
+        values.  Asynchronous, ordered after torch's current stream."""
+        th = self._th()
+        nc = self._env_param_n(name)
+        v = values if isinstance(values, th.Tensor) else th.from_numpy(np.ascontiguousarray(values, np.float64))
+        v = v.to(device=self._device(), dtype=th.float64).contiguous().reshape(-1)
+        idx = self._dev_index(indices)
+        n = v.numel() // nc
+        if v.numel() != n * nc or (idx is not None and idx.numel() != n):
+            raise ValueError(f"{name}: values must be [n] or [n, {nc}] with one row per index")
+        self._order(after_torch=True)
+        check(self._L.b747_set_env_param(self._h, name.encode(), _ptr(v), _ptr(idx), n))
+        self._order(after_torch=False)
+
+    def get_env_param(self, name, indices=None):
+        """float64 device tensor of env indices[k]'s values (default: every env), [n] or [n, 4]; the whole-batch
+        value for every env while the handle is not in per-env mode."""
+        th = self._th()
+        nc = self._env_param_n(name)
+        idx = self._dev_index(indices)
+        n = self.n_envs if idx is None else idx.numel()
+        out = th.full((n, nc) if nc > 1 else (n,), float("nan"), dtype=th.float64, device=self._device())
+        self._order(after_torch=True)
+        check(self._L.b747_get_env_param(self._h, name.encode(), _ptr(idx), n, _ptr(out)))
+        self._order(after_torch=False)
+        return out
+
+    def set_env_param_range(self, name, lo, hi):
+        """From now on every random reset (b747_reset and the in-kernel auto-reset) draws each component of `name`
+        uniformly in [lo, hi].  Enters per-env mode."""
+        nc = self._env_param_n(name)
+        lo = np.ascontiguousarray(np.broadcast_to(np.asarray(lo, np.float64), (nc,)))
+        hi = np.ascontiguousarray(np.broadcast_to(np.asarray(hi, np.float64), (nc,)))
+        dp = ctypes.POINTER(ctypes.c_double)
+        check(self._L.b747_set_env_param_range(self._h, name.encode(), lo.ctypes.data_as(dp), hi.ctypes.data_as(dp), nc))
+
+    def clear_env_param_range(self, name):
+        """`name` keeps each env's current value through later resets."""
+        check(self._L.b747_set_env_param_range(self._h, name.encode(), None, None, self._env_param_n(name)))
 
     # -- episode statistics ---------------------------------------------------------------------
     def episode_stats(self):

@@ -267,7 +267,7 @@ class B747VecEnv(_VecEnvBase):
                  reset_ref_mode=None, disturbance_mode=None, tk=20, sample_time=0.05, action_max=17 * np.pi / 180,
                  vartheta_max=10 * np.pi / 180, use_limiter=False, aero_err=None, reward_config=None, seed=1,
                  dtype=E.F32, device=0, device_tensors=False, env_id_offset=0, monitor=True, copy_outputs=True,
-                 record_capacity=0, track_transfer=False, export_signals=False):
+                 record_capacity=0, track_transfer=False, export_signals=False, param_ranges=None):
         from .core.controller import ResetRefMode
         if reset_ref_mode is None:
             reset_ref_mode = ResetRefMode.CONST  # a VecEnv auto-resets, which needs the random reset
@@ -283,6 +283,9 @@ class B747VecEnv(_VecEnvBase):
             aero_err=aero_err, reward_config=reward_config, seed=seed, auto_reset=True, env_layer=True,
             env_id_offset=env_id_offset, record_capacity=record_capacity, track_transfer=track_transfer,
             export_signals=export_signals)
+        # domain randomisation: {name: (lo, hi)} of the per-env tunables (BatchEngine.ENV_PARAMS), redrawn at every reset
+        for name, (lo, hi) in (param_ranges or {}).items():
+            self.engine.set_env_param_range(name, lo, hi)
         self.num_envs = int(num_envs)
         self.observation_space, self.action_space = make_spaces(observation_type, norm_obs, norm_act, action_max)
         if _VecEnvBase is not object:
@@ -519,6 +522,10 @@ class B747VecEnv(_VecEnvBase):
     def episode_stats(self):
         """(episodes, sum of returns, sum of lengths, sum of squared returns) since the last call."""
         return self.engine.episode_stats()
+
+    def get_env_param(self, name):
+        """Every env's current value of a per-env tunable as a float64 numpy array ([num_envs] or [num_envs, 4])."""
+        return self.engine.get_env_param(name).cpu().numpy()
 
     # ---- checkpoint / resume ----------------------------------------------------------------------------
     def get_state(self):

@@ -165,6 +165,33 @@ int b747_model_initialize(b747_handle *h);
 int b747_set_param(b747_handle *h, const char *name, const double *v, int n);
 int b747_get_param(b747_handle *h, const char *name, double *v, int n);
 
+/* Per-env model tunables: "m0", "Iz", "P", "S", "c_" (1 component each), "PID_SS", "PID_CS" (4 each).  "g" and the
+ * use_* switches stay whole-batch.
+ * The first call of b747_set_env_param or b747_set_env_param_range puts the handle in per-env mode for good: it
+ * allocates one row of doubles per component and env (B747_ERR_ALLOC, handle unchanged, if that fails) and gives every
+ * env the current b747_set_param values.  In per-env mode b747_set_param also writes that name's value of every env,
+ * and b747_get_param returns the whole-batch value.
+ * b747_set_env_param: env env_idx_dev[k] <- values_dev[k][0..n_comp) for k < n (env_idx_dev NULL: env k, n <= n_envs).
+ * b747_get_env_param: out_dev[k][0..n_comp) <- env env_idx_dev[k]'s values (outside per-env mode: the batch value).
+ *   Device arrays; index arrays are int32, an entry outside [0, n_envs) skips k; values must be 8-byte and indices
+ *   4-byte aligned (B747_ERR_ARG before any launch).  Both asynchronous on the handle's stream.
+ * b747_set_env_param_range: host arrays of n_comp bounds; from then on every random reset of an env (b747_reset, masked
+ *   or not, and the auto-reset of the step kernels) draws component j of row r = (index of the name in the list above,
+ *   counting PID_SS / PID_CS components: m0 0, Iz 1, P 2, S 3, c_ 4, PID_SS 5-8, PID_CS 9-12) as
+ *     lo[j] + (hi[j] - lo[j]) * u,  u = the 53-bit uniform of Philox4x32-10 (b747_philox4x32) with key = seed,
+ *     counter = (env id lo, env id hi, episode index, d >> 1), d = 32 + r, words (2 (d & 1), 2 (d & 1) + 1) as
+ *     u = ((w_a >> 5) * 2^26 + (w_b >> 6)) / 2^53,
+ *   with env id = env_id_offset + env and the episode index of that reset -- indices no episode draw uses, so state0,
+ *   reference and aero errors are the same with or without ranges.  lo == hi == NULL removes the range.  B747_ERR_ARG,
+ *   nothing changed, for an unknown name, a wrong n_comp, a bound that is not finite, lo > hi, or a bound <= 0 of m0,
+ *   Iz, S or c_.  Explicit episodes (b747_reset_to*), b747_load_state and resets with B747_RESET_NONE leave every
+ *   env's values as they are, and so does every reset for a name without a range. */
+int b747_set_env_param(b747_handle *h, const char *name, const double *values_dev, const int32_t *env_idx_dev,
+                       int32_t n);
+int b747_get_env_param(b747_handle *h, const char *name, const int32_t *env_idx_dev, int32_t n, double *out_dev);
+int b747_set_env_param_range(b747_handle *h, const char *name, const double *lo_host, const double *hi_host,
+                             int n_comp);
+
 /* Named per-env fields (state, parameters, stage-4 signals) as float64 host arrays [n_envs].
  * Names: the DLL's exported globals ("state" is 6 names state_x..state_wz) plus internal
  * state listed by b747_field_name(). */
@@ -205,7 +232,8 @@ int b747_recorder_read(b747_handle *h, int env, double *out_host, int32_t *n_ste
  * entries of every per-env array the handle allocates, byte for byte -- f32 handles: the double2 and float4 state
  * groups (tick word with its look-up hints, episode index), last_ret, last_len; f64 handles: every slot including
  * state0, tick, flags, ep_idx, last_ret, last_len; both: the exported signals, the transfer tracker and its snapshot,
- * and the recorder rows when the handle has them.  Not in a blob: b747_set_param tunables, the seed, the
+ * and the recorder rows when the handle has them.  Not in a blob: b747_set_param tunables, per-env tunables
+ * (b747_set_env_param; copy them with b747_get_env_param / b747_set_env_param and the same index arrays), the seed, the
  * b747_episode_stats accumulators and the handle's scratch.  After a load, later random resets of env j are drawn
  * from the loading handle's seed, its env_id_offset + j and the episode index that came from the blob.
  * The blob must be 16-byte aligned (cudaMalloc and torch allocations are; a slice at another offset is not), index
