@@ -59,7 +59,8 @@ __device__ __forceinline__ void env_reset64(const DevCfg& c, const double* __res
                                             double* __restrict__ sl, size_t np, int i) {
   int use_ctrl = (c.ctrl_type == B747_CTRL_SEMI_MANUAL || c.ctrl_type == B747_CTRL_FULL_AUTO);
   if (c.reset_ref_mode == B747_RESET_HYBRID) {
-    // Controller._init_model re-creates the Model: per-env tunables back to the DLL defaults
+    // Controller._init_model re-creates the Model: altitude set-point and aero errors back to the DLL defaults.  The
+    // handle's and the env's tunables (PID_SS, PID_CS, P, ...) are configuration and survive (b747.h, b747_set_param)
     use_ctrl = ep.use_ctrl;
     r.h_zh = B747_DEF_H_ZH;
 #pragma unroll

@@ -161,7 +161,11 @@ int b747_model_step(b747_handle *h, int32_t n_steps);
 int b747_model_initialize(b747_handle *h);
 
 /* Whole-batch model tunables (the DLL globals the Python layer never varies per env):
- * "PID_SS"[4], "PID_CS"[4], "P", "Iz", "S", "c_", "g", "m0", "use_RP", "use_RL", "use_PID_SS". */
+ * "PID_SS"[4], "PID_CS"[4], "P", "Iz", "S", "c_", "g", "m0", "use_RP", "use_RL", "use_PID_SS".
+ * These values, and the per-env ones below, are configuration: they survive every reset, HYBRID resets included.  This
+ * differs from the reference, whose HYBRID reset re-creates the Model (Controller._init_model) and so puts PID_SS,
+ * PID_CS, P, use_RP and use_PID_* back to the DLL defaults; at the defaults both behave the same.  A caller who wants
+ * the reference's behaviour sets the defaults (DESIGN.md section 7). */
 int b747_set_param(b747_handle *h, const char *name, const double *v, int n);
 int b747_get_param(b747_handle *h, const char *name, double *v, int n);
 

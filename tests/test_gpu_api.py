@@ -59,6 +59,60 @@ def test_scalar_boundary_bound_like_core_model_py():
     shutil.rmtree(tmp, ignore_errors=True)
 
 
+def test_scalar_boundary_tunables_match_oracle():
+    """The scalar drop-in with every airframe parameter and gain away from its default, written into the exported
+    globals the way core/model.py writes them (in_dll(...).value, array items), and both gain sets acting (use_PID_SS =
+    use_PID_CS = 1): every exported signal against the oracle's model given the same values, 1e-9, over 300 steps."""
+    from b747_rl_ctrl_b200 import _lib
+    from oracle import oracle as O
+    from test_gpu_parity import DDT2, SIG_FIELDS, tuned_params
+    O.build()
+    real_T = ctypes.c_double
+    tmp = tempfile.mkdtemp()
+    path = os.path.join(tmp, "tuned.so")
+    shutil.copyfile(_lib.SCALAR_LIB_PATH, path)
+    dll = ctypes.cdll.LoadLibrary(path)
+    m = O.CModel()
+
+    def glob(name, n=1):
+        return (real_T * n).in_dll(dll, name) if n > 1 else real_T.in_dll(dll, name)
+
+    def put(name, v):
+        v = np.atleast_1d(np.asarray(v, np.float64))
+        if len(v) > 1:
+            arr = glob(name, len(v))
+            for k, x in enumerate(v):
+                arr[k] = float(x)
+        else:
+            glob(name).value = float(v[0])
+        m.set(name, v if len(v) > 1 else v[0])
+
+    for nm, v in tuned_params(O).items():
+        put(nm, v)
+    put("state0", [0.0, 8000.0, 230.0, 2.0, 0.02, 0.0])
+    dll.model_simple_initialize()
+    m.initialize()
+    for nm, v in (("use_PID_SS", 1.0), ("use_PID_CS", 1.0), ("h_zh", 8200.0), ("vartheta", 0.0), ("deltaz", 0.0)):
+        put(nm, v)
+    state = glob("state", 6)
+    worst = {}
+    for k in range(300):
+        dll.model_simple_step()
+        m.step()
+        for name, (oname, idx, floor) in SIG_FIELDS.items():
+            ref = np.atleast_1d(m.get(oname))[idx]
+            got = state[idx] if oname == "state" else glob(oname).value
+            q = abs(got - ref) / max(1e-9 * (abs(ref) + floor), 1e-300)
+            worst[oname + str(idx)] = max(worst.get(oname + str(idx), 0.0), q)
+        _, oname, a, r = DDT2
+        ref = m.get(oname)
+        worst[oname] = max(worst.get(oname, 0.0), abs(glob(oname).value - ref) / (a + r * abs(ref)))
+    print("scalar drop-in, worst signals (deviation / bar):", sorted(worst.items(), key=lambda kv: -kv[1])[:4])
+    assert all(v <= 1.0 for v in worst.values()), {k: v for k, v in worst.items() if not v <= 1.0}
+    assert glob("sim_time").value == pytest.approx(3.0) and abs(glob("U_com_PID").value) > 0
+    shutil.rmtree(tmp, ignore_errors=True)
+
+
 @pytest.mark.parametrize("name", ["K1", "K3", "K4", "K5"])
 def test_model_dropin_matches_dll_kats(name):
     """Model attribute surface (core/model.py) stepping on the GPU vs signals recorded from the DLL."""
@@ -499,7 +553,9 @@ def test_explicit_oscillating_episode_on_canonical_f32_handle(oracle):
 
 def test_step_host_graph_replay_with_pinned_buffers():
     """With pinned host buffers b747_step_host replays its pipeline as a CUDA graph (one launch call per step); results
-    equal the eager pipeline's on pageable buffers, across buffer sets and across a parameter change."""
+    equal the eager pipeline's on pageable buffers, across buffer sets and across parameter changes: set_param, entering
+    per-env mode with a range, per-env values (device rows only) and another range, each redrawn at the 10-step
+    episodes' auto-resets."""
     import torch
     from b747_rl_ctrl_b200 import engine as E
     n = 3000
@@ -511,10 +567,16 @@ def test_step_host_graph_replay_with_pinned_buffers():
     acts = [pin(n) for _ in range(3)]
     obs_p, rew_p, done_p = pin(n, 3), pin(n), pin(n, dt=torch.uint8)
     rng = np.random.default_rng(2)
-    for k in range(24):
-        if k == 12:  # launch arguments change: the captured graphs must not be replayed
-            for e in engs:
+    for k in range(40):
+        for e in engs:
+            if k == 12:  # launch arguments change: the captured graphs must not be replayed
                 e.set_param("P", [2.0e5])
+            elif k == 16:  # per-env mode: the twin kernel and its by-value EnvParams
+                e.set_env_param_range("m0", [2.4e5], [3.4e5])
+            elif k == 23:  # device rows only
+                e.set_env_param("Iz", np.linspace(5.5e7, 7.5e7, n))
+            elif k == 27:  # another by-value EnvParams
+                e.set_env_param_range("PID_SS", [-6.5, -1.4, -7.0, 50.0], [-5.5, -1.1, -6.0, 65.0])
         a = rng.uniform(-1, 1, n).astype(np.float32)
         o0, r0, d0 = engs[0].step_host(a)
         buf = acts[k % 3]

@@ -7,7 +7,8 @@ BatchEngine.set_env_param ..., B747VecEnv(param_ranges=...)).
   * routing: the twins run by template arguments, a canonical handle without per-env mode still runs tier 0;
   * draws: ranged values equal lo + (hi - lo) u with u recomputed from b747_philox4x32 at the documented counter, the
     episode draws do not move, masked resets redraw masked envs only, explicit episodes and loads leave values alone;
-  * against the float64 oracle with drawn airframes and gains;
+  * against the float64 oracle with every per-env component drawn at every reset, the oracle computing the draws
+    itself; tunables survive HYBRID resets (unlike the reference's re-created Model);
   * the API's argument checks, index conventions, set_param broadcasting, the fork recipe and the VecEnv option.
 """
 import ctypes
@@ -22,15 +23,15 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 if HERE not in sys.path:
     sys.path.insert(0, HERE)
 
+from test_gpu_parity import ROW0, TUNED_SCALE  # noqa: E402
+
 pytestmark = pytest.mark.gpu
 
 N_BIG = (1 << 18) + 77
 K5 = dict(sample_time=0.05, tk=1.0)  # 20-step episodes
 NAMES = ("m0", "Iz", "P", "S", "c_", "PID_SS", "PID_CS")
-ROW0 = {"m0": 0, "Iz": 1, "P": 2, "S": 3, "c_": 4, "PID_SS": 5, "PID_CS": 9}
 # multipliers of the whole-batch defaults for the second parameter set (the first set is the defaults themselves)
-SCALE = {"m0": 1.15, "Iz": 0.9, "P": 1.08, "S": 0.97, "c_": 1.03, "PID_SS": [1.2, 0.8, 1.1, 0.9],
-         "PID_CS": [0.8, 1.25, 0.9, 1.1]}
+SCALE = {nm: TUNED_SCALE[nm] for nm in NAMES}
 
 
 def _bits(x):
@@ -222,6 +223,75 @@ def test_f64_model_step_per_env_equals_whole_batch(E):
     assert not np.array_equal(fw[0]["h"], fw[1]["h"]), "the two parameter sets must fly differently"
 
 
+class _Models:
+    """Oracle models of a model-stepping handle, with OracleBatch's gather / ticks (test_gpu_parity._field_ratios)."""
+
+    def __init__(self, models):
+        self.m = models
+
+    def gather(self, name, idx=0):
+        return np.array([np.atleast_1d(m.get(name))[idx] for m in self.m])
+
+    def ticks(self):
+        return np.array([m.tick for m in self.m], np.int64)
+
+
+@pytest.mark.parametrize("per_env", [True, False])
+def test_model_step_tunables_match_oracle(E, per_env):
+    """env_layer = 0 with use_PID_SS = use_PID_CS = 1, so that both gain sets act: b747_model_step with every tunable
+    away from its default -- per env (k_model_step64<true>, values inside tuned_ranges, g set for the batch) or by
+    set_param (k_model_step64<false>, tuned_params) -- against oracle models given the same values: the 16 states,
+    every exported signal and the tick of every env at 1e-9 after every 20 of 400 model steps."""
+    from oracle import oracle as O
+    from test_gpu_parity import _field_ratios, tuned_params, tuned_ranges
+    O.build()
+    n = 256
+    rng = np.random.default_rng(6)
+    tp = tuned_params(O)
+    if per_env:
+        vals = {nm: lo + (hi - lo) * rng.uniform(size=(n, len(lo))) for nm, (lo, hi) in tuned_ranges(O).items()}
+        vals["g"] = np.tile(tp["g"], (n, 1))
+    else:
+        vals = {nm: np.tile(v, (n, 1)) for nm, v in tp.items()}
+    s0 = np.stack([np.zeros(n), rng.uniform(3000, 10000, n), rng.uniform(200, 260, n), rng.uniform(-5, 5, n),
+                   rng.uniform(-0.05, 0.05, n), np.zeros(n)], axis=1)
+    hzh, vzh = s0[:, 1] + rng.uniform(-300, 300, n), rng.uniform(-0.1, 0.1, n)
+    eng = E.BatchEngine(n_envs=n, dtype=E.F64, env_layer=False, export_signals=True, seed=4)
+    for nm, v in vals.items():
+        if per_env and nm != "g":
+            eng.set_env_param(nm, v if E_N(nm) > 1 else v[:, 0])
+        else:
+            eng.set_param(nm, v[0])
+    eng.set_param("use_PID_SS", 1.0)
+    eng.reset()
+    for k, nm in enumerate(("state0_x", "state0_y", "state0_Vx", "state0_Vy", "state0_vartheta", "state0_wz")):
+        eng.set(nm, s0[:, k])
+    eng.model_initialize()
+    eng.set("h_zh", hzh)
+    eng.set("vartheta", vzh)
+    eng.set("deltaz", np.zeros(n))
+    eng.set("flags", (eng.get("flags").astype(np.int64) | 4).astype(np.float64))   # use_PID_CS >= 1 (core/model.py)
+    models = [O.CModel() for _ in range(n)]
+    for i, m in enumerate(models):
+        for nm, v in vals.items():
+            m.set(nm, v[i] if len(v[i]) > 1 else v[i][0])
+        m.set("state0", s0[i])
+        m.initialize()
+        for nm, v in (("h_zh", hzh[i]), ("vartheta", vzh[i]), ("deltaz", 0.0), ("use_PID_SS", 1.0), ("use_PID_CS", 1.0)):
+            m.set(nm, v)
+    ob = _Models(models)
+    ratios = {}
+    for _ in range(20):
+        eng.model_step(20)
+        for m in models:
+            m.step(20)
+        _field_ratios(eng, ob, ratios)
+    print("model step, worst fields (deviation / bar):", sorted(ratios.items(), key=lambda kv: -kv[1])[:4])
+    assert all(v <= 1.0 for v in ratios.values()), {k: v for k, v in ratios.items() if not v <= 1.0}
+    assert np.abs(ob.gather("vartheta_zh")).min() > 0 and np.abs(ob.gather("U_com_PID")).min() > 0  # both loops act
+    eng.close()
+
+
 ROUTING_SCRIPT = r"""
 import json, sys
 import numpy as np
@@ -253,13 +323,26 @@ for tag, kw in cases.items():
 eng = E.BatchEngine(n_envs=256, dtype=E.F64, env_layer=False)
 eng.set_env_param_range("PID_SS", [0.1] * 4, [0.2] * 4)
 out["model"] = names(eng, lambda: eng.model_step(1), sys.argv[2] + "/m.json")
+# test_entering_per_env_mode_mid_run's handles: per-env mode entered after an auto-reset, in the middle of an episode
+for tag, dt in (("midrun", E.F32), ("midrun-f64", E.F64)):
+    eng = E.BatchEngine(n_envs=512, dtype=dt, seed=9, sample_time=0.1, tk=2.0)
+    eng.reset()
+    a = np.zeros(512, eng.np_dtype)
+    for _ in range(29):
+        eng.step_host(a)
+    out[tag + "-batch"] = names(eng, lambda: eng.step_host(a), sys.argv[2] + "/r.json")
+    eng.set_env_param("Iz", np.full(512, 6.0e7))
+    eng.set_env_param_range("P", [2.5e5], [3.0e5])
+    out[tag] = names(eng, lambda: eng.step_host(a), sys.argv[2] + "/s.json")
+    eng.close()
 print(json.dumps(out))
 """
 
 
 def test_routing(E, tmp_path):
     """One profiled launch per case, in a child process (its own profiler session): the twins' template arguments,
-    and tier 0 for a canonical handle without per-env mode."""
+    tier 0 for a canonical handle without per-env mode, and the switch of test_entering_per_env_mode_mid_run's handles
+    (plain kernel after an auto-reset, twin once per-env values and a range arrive mid-episode)."""
     import json
     import subprocess
     want = {
@@ -271,6 +354,10 @@ def test_routing(E, tmp_path):
         "f64-batch": "k_env_step64<false>",
         "f64": "k_env_step64<true>",
         "model": "k_model_step64<true>",
+        "midrun-batch": "k_env_step32<0, 4, false, false>",
+        "midrun": "k_env_step32<5, -1, false, false>",
+        "midrun-f64-batch": "k_env_step64<false>",
+        "midrun-f64": "k_env_step64<true>",
     }
     flags = ["-s"] if sys.flags.no_user_site else []
     r = subprocess.run([sys.executable, *flags, "-c", ROUTING_SCRIPT, os.path.dirname(HERE), str(tmp_path)],
@@ -368,76 +455,117 @@ def test_draws(E, f64):
 
 
 # ---- float64 oracle ------------------------------------------------------------------------------------------------
-ORACLE_FAMILIES = {  # f32 bounds of DESIGN.md 4.2: d obs / (1 + |obs|), d reward
-    "canonical": (dict(), 1e-6, 2e-3),
-    "quality-semi-hybrid": (dict(rew_type=2, ctrl_type=2, reset_ref_mode=2), 5e-4, 2e-3),
+ORACLE_FAMILIES = {  # engine / oracle keywords, engine-only keywords, family of DESIGN.md 4.2 (test_gpu_parity)
+    "canonical": (dict(), None, "K10"),                                                     # tier-1 twin
+    "speed-addproc": (dict(obs_type=1, ctrl_mode=1, action_max=1.0), None, "speed_addproc"),  # PID_SS feeds the elevator
+    "quality-semi-hybrid": (dict(rew_type=2, ctrl_type=2, reset_ref_mode=2), None, "quality_semimanual"),  # tier 2, PID_CS
+    "canonical-full": (dict(), dict(export_signals=True, track_transfer=True, record_capacity=16), "K10"),  # tier-3 twin
 }
 
 
 @pytest.mark.parametrize("fam", list(ORACLE_FAMILIES))
 @pytest.mark.parametrize("f64", [False, True])
 def test_against_oracle(E, fam, f64):
-    """m0 +-20 %, Iz +-20 %, P +-10 %, PID_SS +-30 % drawn at every reset; each oracle instance gets its env's values
-    once per episode (read back after the reset that drew them).  float64: observations within 1e-12 + 1e-9 relative,
-    rewards 1e-10 (test_gpu_parity); f32 twins: the family bounds of DESIGN.md 4.2 inside the flight envelope, with
-    the CLASSIC reward-branch allowance.  Three episodes; the measured maxima are printed."""
+    """All 13 per-env components drawn at every reset (m0, Iz +-20 %, P, S, c_ +-10 %, every PID_SS / PID_CS component
+    0.7-1.3 x its default) and g set for the whole batch.  The oracle computes each env's values itself (lo + (hi - lo) u
+    from its own Philox, episode index counted from its own done flags); the handle's get_env_param equals them bit for
+    bit after every reset.  512 envs, five 10-step episodes.  float64 with signals: observations, rewards, the 16
+    states, every exported signal and the tick at test_gpu_parity's bars; f32 twins: the family bounds of DESIGN.md 4.2
+    inside the flight envelope.  The measured maxima are printed."""
     from oracle import oracle as O
-    from test_gpu_parity import _envelope_update
+    from test_gpu_parity import (F64_OBS_TOL, F64_REW_TOL, FAMILY_BOUNDS, _assert_bound, _f32_bound_rollout,
+                                 _rollout_compare, tuned_params, tuned_ranges)
     O.build()
-    kw, b_obs, b_rew = ORACLE_FAMILIES[fam]
-    n = 512
-    eng = E.BatchEngine(n_envs=n, dtype=E.F64 if f64 else E.F32, seed=9, sample_time=0.05, tk=0.5, **kw)
-    for nm, f in (("m0", 0.2), ("Iz", 0.2), ("P", 0.1)):
-        v = eng.get_param(nm)
-        eng.set_env_param_range(nm, v * (1 - f), v * (1 + f))
-    ss = eng.get_param("PID_SS", 4)
-    eng.set_env_param_range("PID_SS", np.minimum(ss * 0.7, ss * 1.3), np.maximum(ss * 0.7, ss * 1.3))
-    ob = O.OracleBatch(O.make_cfg(seed=9, sample_time=0.05, tk=0.5, **kw), n)
-    eng.reset()
-    ob.reset()
+    kw, ekw, bound = ORACLE_FAMILIES[fam]
+    kw = dict(sample_time=0.05, tk=0.5, **kw)
+    params, ranges = {"g": tuned_params(O)["g"]}, tuned_ranges(O)
+    n, steps = 512, 50
+    if f64:
+        wo, wr, nd, eng = _rollout_compare(E, O, E.F64, n, steps, kw, 9, F64_OBS_TOL, F64_REW_TOL, fields=True, ekw=ekw,
+                                           params=params, ranges=ranges)
+        print(f"oracle {fam} f64: max |d obs| {wo:.3e}, max |d rew| {wr:.3e}")
+        eng.close()
+    else:
+        res = _f32_bound_rollout(E, O, n, steps, kw, 9, ekw=ekw, params=params, ranges=ranges)
+        _assert_bound(f"oracle {fam} twin", res, *FAMILY_BOUNDS[bound])
+        nd = res["n_done"]
+    assert nd == n * steps // 10
 
-    def give(envs):
-        vals = {nm: eng.get_env_param(nm).cpu().numpy() for nm in ("m0", "Iz", "P", "PID_SS")}
-        for i in envs:
-            m = ob.model(int(i))
-            for nm, v in vals.items():
-                m.set(nm, v[i])
 
-    give(range(n))
-    rng = np.random.default_rng(0)
-    out = np.zeros(n, bool)
-    mo = mr = 0.0
-    for k in range(30):  # three episodes
-        a = rng.uniform(-1, 1, n)
-        obs, rew, done = eng.step_host(a.astype(eng.np_dtype))
-        inside = _envelope_update(ob, out, np.zeros(n, bool)) if not f64 else np.ones(n, bool)
-        o_o, r_o, d_o, _ = ob.step(a)
-        assert np.array_equal(done.astype(bool), d_o), f"done flags differ at step {k}"
-        if f64:
-            mo = max(mo, float(np.max(np.abs(obs - o_o) / (1e-3 + np.abs(o_o)))))
-            mr = max(mr, float(np.abs(rew - r_o).max()))
-            assert (np.abs(obs - o_o) <= 1e-12 + 1e-9 * np.abs(o_o)).all(), f"obs beyond 1e-9 at step {k}"
-            assert (np.abs(rew - r_o) <= 1e-10).all(), f"reward beyond 1e-10 at step {k}"
-        else:
-            d_obs = (np.abs(obs - o_o) / (1 + np.abs(o_o))).max(axis=1)
-            bar = np.full(n, b_rew)
-            if eng.cfg.rew_type == E.REW_CLASSIC:  # reward branch at |dvartheta / vf| = 0.05
-                vr = np.where(ob.gather("use_PID_CS") >= 1.0, ob.gather("vartheta_zh"), ob.gather("vartheta"))
-                vf = np.where(vr != 0, vr, eng.cfg.vartheta_max)
-                edge = np.abs(np.abs(ob.gather("dvartheta") / vf) - 0.05) <= 2e-3
-                bar = np.where(edge, b_rew + 0.08, bar)
-            ok = inside | d_o
-            mo = max(mo, float(d_obs[ok].max()))
-            mr = max(mr, float(np.abs(rew - r_o)[ok].max()))
-            bad = ok & ((d_obs > b_obs) | (np.abs(rew - r_o) > bar))
-            assert not bad.any(), (f"{fam}: f32 twin beyond the family bound at step {k}, envs {np.nonzero(bad)[0][:8]}: "
-                                   f"obs {d_obs[bad][:4]}, reward {np.abs(rew - r_o)[bad][:4]}")
-            out &= ~d_o
-        if d_o.any():
-            give(np.nonzero(d_o)[0])
-    print(f"oracle {fam} {'f64' if f64 else 'f32'}: max obs diff {mo:.3e} "
-          f"({'relative' if f64 else '/ (1 + |obs|)'}), max reward diff {mr:.3e}")
+@pytest.mark.parametrize("per_env", [False, True])
+def test_tunables_survive_hybrid_resets(E, per_env):
+    """A HYBRID reset of the reference re-creates its Model with the default gains and thrust (Controller._init_model);
+    the kernels keep the handle's tunables -- set_param values, or set_env_param values of every env -- across every
+    reset.  They read back unchanged after three episodes, the float64 run matches the oracle given them again after
+    each of its HYBRID resets (reapply_after_hybrid_reset), and it does not match an oracle left at its defaults."""
+    from oracle import oracle as O
+    from test_gpu_parity import F64_OBS_TOL, F64_REW_TOL, _rollout_compare, tuned_params, tuned_ranges
+    O.build()
+    kw = dict(rew_type=2, ctrl_type=2, reset_ref_mode=2, sample_time=0.05, tk=0.5)
+    n = 256
+    rng = np.random.default_rng(3)
+    vals = {nm: lo + (hi - lo) * rng.uniform(size=(n, len(lo))) for nm, (lo, hi) in tuned_ranges(O).items()}
+    params = None if per_env else tuned_params(O)
+
+    def give(eng, tun):
+        for nm, v in vals.items():
+            eng.set_env_param(nm, v if E_N(nm) > 1 else v[:, 0])
+            tun.set_env_param(nm, v)
+
+    def run(reapply):
+        return _rollout_compare(E, O, E.F64, n, 30, kw, 9, F64_OBS_TOL, F64_REW_TOL, fields=True, params=params,
+                                at_step={0: give} if per_env else None, reapply_hybrid=reapply)
+
+    _, _, nd, eng = run(True)
+    assert nd == 3 * n
+    if per_env:
+        for nm, v in vals.items():
+            assert _same(eng.get_env_param(nm).cpu().numpy().reshape(n, -1), v), f"{nm} changed by a HYBRID reset"
+    else:
+        for nm, v in params.items():
+            assert _same(np.atleast_1d(eng.get_param(nm, len(v))), v), f"{nm} changed by a HYBRID reset"
     eng.close()
+    with pytest.raises(AssertionError):
+        run(False)
+
+
+@pytest.mark.parametrize("f64", [False, True])
+def test_entering_per_env_mode_mid_run(E, f64):
+    """A canonical K = 10 handle steps through an auto-reset on its plain kernel (f32: tier 0, whose auto-reset writes
+    only the lean state groups, so the twin then reads general groups last written by b747_reset; f64:
+    k_env_step64<false>) and takes per-env values of every name, and ranges of P, PID_SS and PID_CS, in the middle of its
+    second episode.  The oracle takes the same values at the same step and draws the ranged ones at its later resets.
+    Two more episodes against the oracle -- f32: the K10 bound of DESIGN.md 4.2, f64: every field at 1e-9.  That the
+    plain kernel runs before the switch and the twin after it is checked by kernel name in test_routing (one profiler
+    session per process)."""
+    from oracle import oracle as O
+    from test_gpu_parity import (F64_OBS_TOL, F64_REW_TOL, FAMILY_BOUNDS, _assert_bound, _f32_bound_rollout,
+                                 _rollout_compare, tuned_ranges)
+    O.build()
+    kw = dict(sample_time=0.1, tk=2.0)   # 20-step episodes
+    n, switch, steps = 512, 30, 70
+    rng = np.random.default_rng(8)
+    ranges = tuned_ranges(O)
+    vals = {nm: lo + (hi - lo) * rng.uniform(size=(n, len(lo))) for nm, (lo, hi) in ranges.items()}
+
+    def enter(eng, tun):
+        for nm, v in vals.items():
+            eng.set_env_param(nm, v if E_N(nm) > 1 else v[:, 0])
+            tun.set_env_param(nm, v)
+        for nm in ("P", "PID_SS", "PID_CS"):
+            eng.set_env_param_range(nm, *ranges[nm])
+            tun.set_range(nm, *ranges[nm])
+
+    if f64:
+        wo, wr, nd, eng = _rollout_compare(E, O, E.F64, n, steps, kw, 9, F64_OBS_TOL, F64_REW_TOL, fields=True,
+                                           at_step={switch: enter})
+        eng.close()
+        print(f"f64 entering per-env mode at step {switch}: max |d obs| {wo:.3e}, max |d rew| {wr:.3e}")
+    else:
+        res = _f32_bound_rollout(E, O, n, steps, kw, 9, at_step={switch: enter})
+        _assert_bound(f"tier 0 -> twin at step {switch}", res, *FAMILY_BOUNDS["K10"])
+        nd = res["n_done"]
+    assert nd == 3 * n
 
 
 # ---- API -----------------------------------------------------------------------------------------------------------

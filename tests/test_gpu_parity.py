@@ -88,17 +88,142 @@ def _field_ratios(eng, ob, ratios, ddt_scale=1.0, inside=None):
     assert np.array_equal(eng.get("tick").astype(np.int64), ob.ticks()), "model tick counters differ"
 
 
+# ---- tunables away from their defaults --------------------------------------------------------------------------------
+# Airframe parameters and PID gains are settable per handle (b747_set_param) and, all but g, per env
+# (b747_set_env_param / b747_set_env_param_range).  A kernel that read a default instead of the tunable at one site would
+# agree with the oracle at the defaults, so the families below also run at these values.
+TUNABLES = ("m0", "Iz", "P", "S", "c_", "g", "PID_SS", "PID_CS")
+ROW0 = {"m0": 0, "Iz": 1, "P": 2, "S": 3, "c_": 4, "PID_SS": 5, "PID_CS": 9}   # per-env rows, include/b747.h
+# batch-wide values: multipliers of the defaults
+TUNED_SCALE = {"m0": 1.15, "Iz": 0.9, "P": 1.08, "S": 0.97, "c_": 1.03, "g": 0.998, "PID_SS": [1.2, 0.8, 1.1, 0.9],
+               "PID_CS": [0.8, 1.25, 0.9, 1.1]}
+# per-env ranges: default x (1 -+ f), every PID component ordered for its sign
+RANGE_FRAC = {"m0": 0.2, "Iz": 0.2, "P": 0.1, "S": 0.1, "c_": 0.1, "PID_SS": 0.3, "PID_CS": 0.3}
+
+
+def tunable_defaults(O):
+    """The DLL defaults, as the oracle's model holds them."""
+    m = O.CModel()
+    return {nm: np.atleast_1d(np.asarray(m.get(nm), np.float64)) for nm in TUNABLES}
+
+
+def tuned_params(O):
+    d = tunable_defaults(O)
+    return {nm: d[nm] * np.asarray(TUNED_SCALE[nm]) for nm in TUNABLES}
+
+
+def tuned_ranges(O):
+    d = tunable_defaults(O)
+    out = {}
+    for nm, f in RANGE_FRAC.items():
+        a, b = d[nm] * (1 - f), d[nm] * (1 + f)
+        out[nm] = (np.minimum(a, b), np.maximum(a, b))
+    return out
+
+
+class OracleTunables:
+    """The tunables of every env of an OracleBatch, kept as the handle under test keeps its own: whole-batch values
+    (set_param), per-env values (set_env_param) and ranges drawn at every random reset by the formula of include/b747.h,
+    lo + (hi - lo) u with u = the oracle's b747o_uniform53(seed, env id, episode, 32 + row).  The episode index of each
+    env is counted from the ORACLE's done flags, so no input of the oracle is read back from the handle under test."""
+
+    def __init__(self, O, ob, cfg_o, env_id_offset=0, reapply_hybrid=True):
+        self._L, self.ob, self.seed = O.olib(), ob, cfg_o.seed
+        self.hybrid = cfg_o.reset_ref_mode == O.RESET_HYBRID
+        self.reapply_hybrid = reapply_hybrid
+        self.ids = env_id_offset + np.arange(ob.n)
+        self.epi = np.zeros(ob.n, np.int64)
+        self.vals = {nm: np.tile(v, (ob.n, 1)) for nm, v in tunable_defaults(O).items()}
+        self.ranges = {}
+
+    def set_param(self, name, v):
+        """b747_set_param: the batch value, and in per-env mode every env's value of that name."""
+        self.vals[name] = np.tile(np.atleast_1d(np.asarray(v, np.float64)), (self.ob.n, 1))
+        self._give(range(self.ob.n), [name])
+
+    def set_env_param(self, name, v):
+        self.vals[name] = np.asarray(v, np.float64).reshape(self.ob.n, -1).copy()
+        self._give(range(self.ob.n), [name])
+
+    def set_range(self, name, lo, hi):
+        self.ranges[name] = tuple(np.atleast_1d(np.asarray(x, np.float64)) for x in (lo, hi))
+
+    def _give(self, envs, names=None):
+        for i in envs:
+            m = self.ob.model(int(i))
+            for nm in names if names is not None else self.vals:
+                v = self.vals[nm][i]
+                m.set(nm, v if len(v) > 1 else v[0])
+
+    def reset(self):
+        """After ob.reset(): episode 0 of every env."""
+        self.epi[:] = 0
+        self._on_reset(np.arange(self.ob.n))
+
+    def step(self, d_o):
+        """After ob.step(): the envs that finished started their next episode."""
+        envs = np.nonzero(d_o)[0]
+        self.epi[envs] += 1
+        self._on_reset(envs)
+
+    def _on_reset(self, envs):
+        for nm, (lo, hi) in self.ranges.items():
+            for i in envs:
+                for j in range(len(lo)):
+                    u = self._L.b747o_uniform53(self.seed, int(self.ids[i]), int(self.epi[i]), 32 + ROW0[nm] + j)
+                    self.vals[nm][i, j] = lo[j] + (hi[j] - lo[j]) * u
+        if self.ranges:
+            self._give(envs, list(self.ranges))
+        if self.hybrid and self.reapply_hybrid:
+            reapply_after_hybrid_reset(self, envs)
+
+    def check_handle(self, eng, envs=None):
+        """get_env_param of the handle equals the values the oracle flies, bit for bit."""
+        envs = np.arange(self.ob.n) if envs is None else np.asarray(envs)
+        for nm in self.ranges:
+            got = eng.get_env_param(nm).cpu().numpy().reshape(self.ob.n, -1)[envs]
+            want = self.vals[nm][envs]
+            assert np.array_equal(got.view(np.uint64), want.view(np.uint64)), \
+                f"{nm}: handle values differ from lo + (hi - lo) u of the oracle's draw"
+
+
+def reapply_after_hybrid_reset(tun, envs):
+    """A HYBRID reset of the reference re-creates its Model (Controller._init_model; oracle/b747_env_ref.c), which puts
+    PID_SS, PID_CS, P and the use_* switches back to the DLL defaults.  The kernels keep the handle's and every env's
+    tunables across every reset: they are configuration (include/b747.h at b747_set_param, DESIGN.md section 7).  So
+    the oracle is given the handle's values again after each of its HYBRID resets."""
+    tun._give(envs)
+
+
+def _with_tunables(O, eng, ob, cfg_o, params=None, ranges=None, reapply_hybrid=True):
+    """Apply batch-wide `params` and per-env `ranges` to the handle and build the oracle's side of them."""
+    tun = OracleTunables(O, ob, cfg_o, reapply_hybrid=reapply_hybrid)
+    for nm, v in (params or {}).items():
+        eng.set_param(nm, v)
+        tun.set_param(nm, v)
+    for nm, (lo, hi) in (ranges or {}).items():
+        eng.set_env_param_range(nm, lo, hi)
+        tun.set_range(nm, lo, hi)
+    return tun
+
+
 def _rollout_compare(E, O, dtype, n, steps, kw, seed, obs_tol, rew_tol, sticky=0, fields=False, ddt_scale=1.0,
-                     max_excused=0.02):
+                     max_excused=0.02, params=None, ranges=None, at_step=None, reapply_hybrid=True, ekw=None):
     """Step engine and oracle in lock-step with the same actions; every env is held to the tolerance at every step
     inside the flight envelope (max_excused: largest share of env-steps outside it).  Done flags,
-    step counts and tick counters are compared for all envs.  Returns the worst deviations."""
+    step counts and tick counters are compared for all envs.  Returns the worst deviations.
+    params: batch-wide tunables, ranges: per-env ranges, both given to the handle and to every oracle env;
+    at_step: {k: fn(eng, tun)} called before step k; ekw: engine-only keywords."""
     cfg_o = O.make_cfg(seed=seed, **kw)
-    eng = E.BatchEngine(n_envs=n, dtype=dtype, seed=seed, auto_reset=True, export_signals=fields, **kw)
+    eng = E.BatchEngine(n_envs=n, dtype=dtype, seed=seed, auto_reset=True, **{"export_signals": fields, **(ekw or {})},
+                        **kw)
     ob = O.OracleBatch(cfg_o, n)
+    tun = _with_tunables(O, eng, ob, cfg_o, params, ranges, reapply_hybrid)
     ratios = {}
     eng.reset()
     o0 = ob.reset()
+    tun.reset()
+    tun.check_handle(eng)
     assert (o0 == 0).all()
     rng = np.random.default_rng(seed)
     amax = 1.0 if cfg_o.norm_act else cfg_o.action_max
@@ -112,10 +237,15 @@ def _rollout_compare(E, O, dtype, n, steps, kw, seed, obs_tol, rew_tol, sticky=0
             pass  # hold the previous action: drives the airframe far out of the trimmed envelope
         else:
             a = rng.uniform(-amax, amax, n).astype(eng.np_dtype)
+        if at_step and k in at_step:
+            at_step[k](eng, tun)
         obs, rew, done, term = eng.step_host(a, terminal_obs=term)
         o_o, r_o, d_o, t_o = ob.step(a.astype(np.float64))
         assert np.array_equal(done.astype(bool), d_o), f"done flags differ at step {k}"
         n_done += int(d_o.sum())
+        if d_o.any():
+            tun.step(d_o)
+            tun.check_handle(eng, np.nonzero(d_o)[0])
         ins = _envelope_update(ob, out, d_o)
         excused += int(out.sum())
         eo = np.abs(obs.astype(np.float64) - o_o)[ins]
@@ -168,14 +298,18 @@ def _reward_edge(O, cfg_o, ob, t_o, d_o):
     return edge
 
 
-def _f32_bound_rollout(E, O, n, steps, kw, seed, sticky=0):
+def _f32_bound_rollout(E, O, n, steps, kw, seed, sticky=0, ekw=None, params=None, ranges=None, at_step=None):
     """f32 engine against the oracle; returns per-step worst deviations inside the envelope and the bookkeeping the
-    bound tests assert on.  Done flags are compared bit for bit for ALL envs, excused or not."""
+    bound tests assert on.  Done flags are compared bit for bit for ALL envs, excused or not.  ekw: engine-only
+    keywords; params, ranges, at_step: as in _rollout_compare."""
     cfg_o = O.make_cfg(seed=seed, **kw)
-    eng = E.BatchEngine(n_envs=n, dtype=E.F32, seed=seed, auto_reset=True, **kw)
+    eng = E.BatchEngine(n_envs=n, dtype=E.F32, seed=seed, auto_reset=True, **kw, **(ekw or {}))
     ob = O.OracleBatch(cfg_o, n)
+    tun = _with_tunables(O, eng, ob, cfg_o, params, ranges)
     eng.reset()
     ob.reset()
+    tun.reset()
+    tun.check_handle(eng)
     rng = np.random.default_rng(seed)
     amax = 1.0 if cfg_o.norm_act else cfg_o.action_max
     out = np.zeros(n, bool)                      # env left the envelope in its running episode
@@ -185,10 +319,15 @@ def _f32_bound_rollout(E, O, n, steps, kw, seed, sticky=0):
     for k in range(steps):
         if not (sticky and k % sticky):
             a = rng.uniform(-amax, amax, n).astype(np.float32)
+        if at_step and k in at_step:
+            at_step[k](eng, tun)
         obs, rew, done, term = eng.step_host(a, terminal_obs=term)
         o_o, r_o, d_o, t_o = ob.step(a.astype(np.float64))
         assert np.array_equal(done.astype(bool), d_o), f"done flags differ at step {k}"
         assert np.isfinite(obs).all() and np.isfinite(rew).all()
+        if d_o.any():
+            tun.step(d_o)
+            tun.check_handle(eng, np.nonzero(d_o)[0])
         res["n_done"] += int(d_o.sum())
         inside = _envelope_update(ob, out, d_o)
         eo = (np.abs(term.astype(np.float64) - t_o) / (1.0 + np.abs(t_o))).max(axis=1)   # relative to 1 + |obs|
@@ -251,10 +390,26 @@ VARIANTS = {
 }
 
 
-@pytest.mark.parametrize("name", sorted(VARIANTS))
+# Families run with every airframe parameter and PID gain away from its default (tuned_params: set_param on the handle and
+# on every oracle env): name -> (family of VARIANTS or "canonical", engine-only keywords).
+TUNED = {
+    "tuned_canonical": ("canonical", None),
+    "tuned_K10": ("K10", None),
+    "tuned_K1_tk3": ("K1_tk3", None),
+    "tuned_speed_addproc": ("speed_addproc", None),
+    "tuned_quality_semimanual": ("quality_semimanual", None),
+    "tuned_canonical_full": ("canonical", dict(export_signals=True, track_transfer=True, record_capacity=16)),
+}
+TUNED_F64 = ["tuned_canonical", "tuned_speed_addproc", "tuned_quality_semimanual"]
+TUNED_F32 = ["tuned_K10", "tuned_K1_tk3", "tuned_speed_addproc", "tuned_quality_semimanual", "tuned_canonical_full"]
+
+
+@pytest.mark.parametrize("name", sorted(VARIANTS) + TUNED_F64)
 def test_f64_variants_match_oracle(E, oracle, name):
-    kw = VARIANTS[name]
-    steps = 320 if name == "K1_tk3" else 420
+    fam = TUNED[name][0] if name in TUNED else name
+    kw = VARIANTS.get(fam, {})
+    params = tuned_params(oracle) if name in TUNED else None
+    steps = 320 if fam == "K1_tk3" else 420
     # un-normalised observations carry raw magnitudes (Vx ~ 250): relative bar only
     # Aero disturbance N(-+0.1, 0.5) on the five coefficients makes some members of this family open-loop unstable: a few
     # leave the flight envelope and tumble (excused from there to their next reset, at most 5 % of the env-steps), and the
@@ -262,9 +417,10 @@ def test_f64_variants_match_oracle(E, oracle, name):
     # 4e-14 on these envs within one episode, tools/family_probe.py `dll`), which the two finite-difference signals
     # multiply by 1/h = 100 and 1/h^2.  States and every other signal keep the 1e-9 bar; the floors of dvartheta_dt /
     # dvartheta_dt_dt are widened by 1/h for this family only (measured round 2: 6.7x / 19x the canonical floors).
-    dist = name == "state_angvel_hybrid_dist"
+    dist = fam == "state_angvel_hybrid_dist"
     wo, wr, nd, _ = _rollout_compare(E, oracle, E.F64, 512, steps, kw, 9, F64_OBS_TOL, F64_REW_TOL, fields=True,
-                                     ddt_scale=100.0 if dist else 1.0, max_excused=0.05 if dist else 0.02)
+                                     ddt_scale=100.0 if dist else 1.0, max_excused=0.05 if dist else 0.02,
+                                     params=params)
     assert nd >= 512
     print(f"f64 {name}: max|dobs|={wo:.2e} max|drew|={wr:.2e} episodes={nd}")
 
@@ -340,12 +496,13 @@ FAMILY_BOUNDS = {
 }
 
 
-@pytest.mark.parametrize("name", sorted(VARIANTS))
+@pytest.mark.parametrize("name", sorted(VARIANTS) + TUNED_F32)
 def test_f32_variants_within_bound(E, oracle, name):
-    kw = VARIANTS[name]
-    steps = 320 if name == "K1_tk3" else 420
-    ob, rb, ex = FAMILY_BOUNDS[name]
-    res = _f32_bound_rollout(E, oracle, 512, steps, kw, 9)
+    fam, ekw = TUNED.get(name, (name, None))
+    kw = VARIANTS.get(fam, {})
+    steps = 320 if fam == "K1_tk3" else 420
+    ob, rb, ex = FAMILY_BOUNDS["K10" if fam == "canonical" else fam]
+    res = _f32_bound_rollout(E, oracle, 512, steps, kw, 9, ekw=ekw, params=tuned_params(oracle) if name in TUNED else None)
     assert res["n_done"] >= 512
     _assert_bound(name, res, ob, rb, max_excused=ex)
 

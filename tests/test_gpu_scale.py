@@ -12,7 +12,9 @@ ragged.  For every reachable instantiation (TIER, SW, STG, PFA) this module
   * replays the episode bookkeeping on the host (ep_return += (double)rew in step order) against last_episode() and
     episode_stats();
   * compares three 256-env slices with the float64 oracle -- the first envs, the first tiles the counter hands out and
-    the ragged tail -- under test_gpu_parity's per-family bounds and flight-envelope excusal.
+    the ragged tail -- under test_gpu_parity's per-family bounds and flight-envelope excusal, also with the airframe
+    parameters and gains away from their defaults (batch-wide on tier 0, drawn per env at every reset on the tier 1 and 2
+    twins).
 """
 import json
 import math
@@ -26,7 +28,8 @@ import pytest
 HERE = os.path.dirname(os.path.abspath(__file__))
 if HERE not in sys.path:
     sys.path.insert(0, HERE)
-from test_gpu_parity import FAMILY_BOUNDS, REW_JUMP, _envelope_update, _reward_edge  # noqa: E402
+from test_gpu_parity import (FAMILY_BOUNDS, REW_JUMP, OracleTunables, _envelope_update, _reward_edge,  # noqa: E402
+                              tuned_params, tuned_ranges)
 
 pytestmark = pytest.mark.gpu
 
@@ -45,21 +48,28 @@ SWITCH_BOUNDS = {
     "T1-SW": (1e-6, 1.2e-5, 0.02),
 }
 
-# config -> engine / oracle keywords, engine-only keywords, set_param applied to the handles and every oracle env,
-# the entry points stepped in the multi-tile form with the kernel each must launch (TIER, SW, STG, PFA), bounds
+# config -> engine / oracle keywords, engine-only keywords, set_param values applied to the handles and every oracle env
+# (param; tuned: test_gpu_parity.tuned_params, every airframe parameter and gain away from its default), per-env ranges
+# drawn at every reset (ranges: test_gpu_parity.tuned_ranges; the oracle slices draw the same values on the host), the
+# entry points stepped in the multi-tile form with the kernel each must launch (TIER, SW, STG, PFA), bounds
 CASES = {
     "T0-K1": dict(kw=K1, forms={"step": (0, SW_RP, 1, 0), "packed": (0, SW_RP, 1, 0), "host_packed": (0, SW_RP, 0, 1)},
                   bounds=FAMILY_BOUNDS["K1_tk3"]),
     "T0": dict(kw=K5, forms={"step": (0, SW_RP, 0, 0)}, bounds=FAMILY_BOUNDS["K10"]),
-    "T0-SW": dict(kw=K5, param=("use_RP", 0.0), forms={"step": (0, -1, 0, 0)}, bounds=SWITCH_BOUNDS["T0-SW"]),
+    "T0-SW": dict(kw=K5, param={"use_RP": 0.0}, forms={"step": (0, -1, 0, 0)}, bounds=SWITCH_BOUNDS["T0-SW"]),
     "T1": dict(kw=dict(obs_type=1, ctrl_mode=1, action_max=1.0, **K5), forms={"step": (1, SW_RP, 0, 0)},
                bounds=FAMILY_BOUNDS["speed_addproc"]),
-    "T1-SW": dict(kw=dict(obs_type=1, ctrl_mode=1, action_max=1.0, **K5), param=("use_RL", 1.0),
+    "T1-SW": dict(kw=dict(obs_type=1, ctrl_mode=1, action_max=1.0, **K5), param={"use_RL": 1.0},
                   forms={"step": (1, -1, 0, 0)}, bounds=SWITCH_BOUNDS["T1-SW"]),
     "T2": dict(kw=dict(rew_type=2, ctrl_type=2, reset_ref_mode=2, **K5), forms={"step": (2, -1, 0, 0)},
                bounds=FAMILY_BOUNDS["quality_semimanual"]),
     "T3": dict(kw=K5, ekw=dict(export_signals=True, track_transfer=True, record_capacity=12),
                forms={"step": (3, -1, 0, 0)}, bounds=FAMILY_BOUNDS["K10"]),
+    "T0-TUN": dict(kw=K5, tuned=True, forms={"step": (0, SW_RP, 0, 0)}, bounds=FAMILY_BOUNDS["K10"]),
+    "T1-PE": dict(kw=dict(obs_type=1, ctrl_mode=1, action_max=1.0, **K5), ranges=True, forms={"step": (5, -1, 0, 0)},
+                  bounds=FAMILY_BOUNDS["speed_addproc"]),
+    "T2-PE": dict(kw=dict(rew_type=2, ctrl_type=2, reset_ref_mode=2, **K5), ranges=True, forms={"step": (6, -1, 0, 0)},
+                  bounds=FAMILY_BOUNDS["quality_semimanual"]),
 }
 BOOK_FIELDS = ("tick", "flags", "ep_idx", "last_ret", "last_len")
 
@@ -124,18 +134,28 @@ class Run:
     the single-tile form, the bookkeeping read back from each handle, the oracle deviations per slice."""
 
 
-def _make(E, name, n_chunks=None):
+def _tunables(O, name):
+    """(set_param values, per-env ranges) of a configuration."""
+    c = CASES[name]
+    params = {**(tuned_params(O) if c.get("tuned") else {}), **c.get("param", {})}
+    return params, tuned_ranges(O) if c.get("ranges") else {}
+
+
+def _make(E, name, tun, n_chunks=None):
     c = CASES[name]
     eng = E.BatchEngine(n_envs=N, dtype=E.F32, seed=17, auto_reset=True, **c["kw"], **c.get("ekw", {}))
-    if "param" in c:
-        eng.set_param(c["param"][0], [c["param"][1]])
+    params, ranges = tun
+    for nm, v in params.items():
+        eng.set_param(nm, v)
+    for nm, (lo, hi) in ranges.items():
+        eng.set_env_param_range(nm, lo, hi)
     if n_chunks:
         eng.set_host_chunks(n_chunks)
     eng.reset()
     return eng
 
 
-def _step_forms(E, name, acts, tmp):
+def _step_forms(E, name, tun, acts, tmp):
     """Multi-tile forms: {form: (handle, kernel events of the profiled first step, host history)}."""
     import torch
     dev = torch.device("cuda")
@@ -144,7 +164,7 @@ def _step_forms(E, name, acts, tmp):
     torch.cuda.synchronize()
     out = {}
     for form in c["forms"]:
-        eng = _make(E, name)
+        eng = _make(E, name, tun)
         od, rf, nw = eng.obs_dim, eng.record_floats, (N + 31) // 32
         if form == "step":
             obs = torch.empty(STEPS, N, od, device=dev)
@@ -202,7 +222,7 @@ def _fields(eng):
     return got
 
 
-def _oracle_slices(O, name, acts, hist, resident):
+def _oracle_slices(O, name, tun, acts, hist, resident):
     """Worst deviations of three 256-env slices of the multi-tile run from the float64 oracle."""
     c = CASES[name]
     cfg_o = O.make_cfg(seed=17, **c["kw"])
@@ -211,9 +231,12 @@ def _oracle_slices(O, name, acts, hist, resident):
         m = 256
         ob = O.OracleBatch(cfg_o, m, env_id_offset=lo)
         ob.reset()
-        if "param" in c:
-            for i in range(m):
-                ob.model(i).set(*c["param"])
+        ot = OracleTunables(O, ob, cfg_o, env_id_offset=lo)
+        for nm, v in tun[0].items():
+            ot.set_param(nm, v)
+        for nm, (a, b) in tun[1].items():
+            ot.set_range(nm, a, b)
+        ot.reset()
         out = np.zeros(m, bool)
         r = dict(lo=lo, obs=0.0, rew=0.0, rew_edge=0.0, excused=0, total=0, done_diff=[], n_done=0)
         for k in range(STEPS):
@@ -221,6 +244,8 @@ def _oracle_slices(O, name, acts, hist, resident):
             if not np.array_equal(hist["done"][k, lo:lo + m].astype(bool), d_o):
                 r["done_diff"].append(k)
             r["n_done"] += int(d_o.sum())
+            if d_o.any():
+                ot.step(d_o)
             inside = _envelope_update(ob, out, d_o)
             eo = (np.abs(hist["term"][k, lo:lo + m].astype(np.float64) - t_o) / (1.0 + np.abs(t_o))).max(axis=1)
             er = np.abs(hist["rew"][k, lo:lo + m].astype(np.float64) - r_o)
@@ -245,10 +270,11 @@ def run(request, oracle, tmp_path_factory):
     acts = np.random.default_rng(29).uniform(-1.0, 1.0, (STEPS, N)).astype(np.float32)
     R = Run()
     R.name = name
-    forms = _step_forms(E, name, acts, tmp_path_factory.mktemp(name))
+    tun = _tunables(oracle, name)
+    forms = _step_forms(E, name, tun, acts, tmp_path_factory.mktemp(name))
     R.kernels = {f: ev for f, (_, ev, _) in forms.items()}
     # single-tile form: every chunk launch gives each warp at most one tile
-    ref = _make(E, name, n_chunks=SINGLE_TILE_CHUNKS)
+    ref = _make(E, name, tun, n_chunks=SINGLE_TILE_CHUNKS)
     od = ref.obs_dim
     R.diffs = []
     hist_b = dict(obs=[], rew=[], done=[], term=[])
@@ -303,7 +329,7 @@ def run(request, oracle, tmp_path_factory):
     # oracle on slices of the (first) multi-tile form
     R.resident = resident
     hist = forms[first][2]
-    R.oracle = _oracle_slices(oracle, name, acts, hist, resident) if resident else {}
+    R.oracle = _oracle_slices(oracle, name, tun, acts, hist, resident) if resident else {}
     for f, (eng, _, _) in forms.items():
         eng.close()
     ref.close()
